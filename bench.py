@@ -2,6 +2,7 @@
 """bench.py -- loss-path frames/s, forward + backward, @192x640 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape 192x640|375x1242] [--mode T]
+                    [--dump-outputs DIR]
 
 A *step* is one pass of the whole configured loss path over one batch: `Loss.forward` (all scales, both
 source frames: epipolar map + post-processing, flow warp, SSIM + L1, smoothness, consistency, min mask) followed
@@ -33,6 +34,7 @@ import torch  # noqa: E402
 
 METRIC = "loss-path frames/s fwd+bwd @192x640"
 L2_BYTES = 126 * 1024 * 1024
+DUMP_BYTES = 64 * 10 ** 6
 
 
 def parse():
@@ -56,7 +58,16 @@ def parse():
     ap.add_argument("--no-train-step", action="store_true", help="skip the short whole-train-step measurement (configs[2])")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the DS / DC / 375x1242 lines (BASELINE configs[3], [4])")
     ap.add_argument("--train-steps", type=int, default=30)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss terms and gradients of the last timed step as DIR/<name>.npy "
+                         "(float32; an array is replaced by a fixed seeded sample of its elements when all of them would "
+                         "exceed %d MB); with several GPUs, rank 0's step" % (DUMP_BYTES // 10 ** 6))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 FLOW_DESC = {"iid": "normalised flow ~ N(0, 0.05^2) i.i.d. per pixel (+-32 px at 640: stress case, no locality in the warp gather)",
@@ -306,16 +317,18 @@ class Workload:
             self.dev_sets.append((to(inputs), to(flows, True), to(mobiles, True), to(cams, True), inst_d))
 
     def step_on(self, s):
+        """One forward + backward on input set `s`; returns the losses dict (the gradients land in the leaves' .grad)."""
         inputs, flows, mobiles, cams, inst = s
         for d in (flows, mobiles, cams):
             for v in d.values():
                 v.grad = None
         _, losses = self.loss_mod(inputs, self.ids, flows, mobiles, inst, list(self.scales), cams)
         losses["loss"].backward()
-        return losses["loss"]
+        return losses
 
     def timed_steps(self, dev_sets, steps, warmup, ramp_s):
-        """fwd+bwd steps replayed from CUDA graphs over rotating input sets; returns (total ms, graph_ok)."""
+        """fwd+bwd steps replayed from CUDA graphs over rotating input sets; returns (total ms, graph_ok).
+        `self.last_step` is left as (input set, losses dict) of the last timed step."""
         import torch.distributed as dist
         step_on, world, dev = self.step_on, self.world, self.dev
         for s in dev_sets:   # eager warm-up (also sets the kernel attributes outside any capture)
@@ -337,7 +350,7 @@ class Workload:
                 torch.cuda.synchronize()
                 group = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(group):
-                    outs = [step_on(s) for s in dev_sets]   # noqa: F841
+                    outs = [step_on(s) for s in dev_sets]
                 for s in dev_sets[:r]:
                     g = torch.cuda.CUDAGraph()
                     with torch.cuda.graph(g):
@@ -352,9 +365,10 @@ class Workload:
         def run_rotation():
             if graph_ok:
                 group.replay()
-            else:
-                for s in dev_sets:
-                    step_on(s)
+                return outs[-1]
+            for s in dev_sets:
+                losses = step_on(s)
+            return losses
 
         # clock ramp (untimed) so a short timed region does not run at idle clocks
         t_end = time.perf_counter() + ramp_s
@@ -369,14 +383,16 @@ class Workload:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(q):                      # q * n_sets + r == steps, exactly
-            run_rotation()
+            last = run_rotation()
         for i in range(r):
             if graph_ok:
                 singles[i][0].replay()
+                last = singles[i][1]
             else:
-                step_on(dev_sets[i])
+                last = step_on(dev_sets[i])
         e1.record()
         torch.cuda.synchronize()
+        self.last_step = (dev_sets[r - 1] if r else dev_sets[-1], last)
         ms = e0.elapsed_time(e1)
         if world > 1:
             t = torch.tensor([ms], device=dev)
@@ -465,6 +481,35 @@ class Workload:
         return roof
 
 
+def dump_outputs(directory, last_step):
+    """Writes what one step of the loss path hands its caller -- the loss terms and d/dflow, d/dmobile, d/dpose -- as
+    float32 `directory/<name>.npy`, so that two builds run with the same arguments can be compared output for output.
+    When the gradients together exceed DUMP_BYTES, each one larger than 4096 elements is replaced by the same fixed
+    fraction of its elements, taken at indices drawn (sorted) from numpy's default_rng(0): the same indices in every run."""
+    import numpy as np
+    (_, flows, mobiles, cams, _), losses = last_step
+    tag = lambda v: str(v).replace("-", "m")
+    arrays = {("loss" if k == "loss" else "loss_" + k): v for k, v in losses.items() if torch.is_tensor(v)}
+    for prefix, d in (("grad_flow", flows), ("grad_mobile", mobiles)):
+        for (_, i, s), v in d.items():
+            arrays["%s_%s_s%d" % (prefix, tag(i), s)] = v.grad
+    for i, v in cams.items():
+        arrays["grad_cam_%s" % tag(i)] = v.grad
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    large = {k for k, a in arrays.items() if a.size > 4096}
+    large_bytes = sum(arrays[k].nbytes for k in large)
+    small_bytes = sum(a.nbytes for a in arrays.values()) - large_bytes
+    headers = 1024 * len(arrays)     # an .npy header takes 128 bytes for arrays of this rank; the files stay under the cap
+    keep = min(1.0, (DUMP_BYTES - headers - small_bytes) / max(large_bytes, 1))
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        if keep < 1.0 and k in large:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, int(a.size * keep), replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(directory, k + ".npy"), a)
+    return keep
+
+
 def host_copy_ceiling(dev, world, nbytes=256 << 20, reps=4):
     """Pinned host -> device bandwidth of plain `reps` x 256 MB cudaMemcpyAsync on every rank AT THE SAME TIME (GB/s of this
     rank, min over ranks): what the host's PCIe / memory system gives the e2e upload when all ranks pull together.
@@ -550,6 +595,10 @@ def run_ours(args):
     ms_per_step = ms / args.steps
     value = world * B * args.steps / (ms * 1e-3)
     clocks_now = sampler.summary()
+    if args.dump_outputs and rank == 0:
+        keep = dump_outputs(args.dump_outputs, wl.last_step)
+        print("bench: last timed step's outputs written to %s%s" % (
+            args.dump_outputs, "" if keep == 1.0 else " (gradients sampled: %.3g of their elements)" % keep), file=sys.stderr)
 
     # ---- dominant kernel alone
     roofline = wl.kernel_alone(200, clocks_now.get("sm_mhz"))
@@ -594,7 +643,7 @@ def run_ours(args):
                     inputs_i[kk] = from_frames(fr)
                 pyramid.add_pyramid_levels(inputs_i, [0] + ids, list(scales), packed_sources=packed)
                 inst_i = [{"instances": synthetic.SyntheticInstances(v[5][("inst", j)])} for j in range(len(v[5]))] if with_inst else None
-                loss = step_on((inputs_i, leaf(v[2]), leaf(v[3]), leaf(v[4]), inst_i))
+                loss = step_on((inputs_i, leaf(v[2]), leaf(v[3]), leaf(v[4]), inst_i))["loss"]
                 st.release(i)
                 host_loss.copy_(loss.detach(), non_blocking=True)
         return st, run

@@ -61,6 +61,13 @@ def netinit_inputs(B=2, H=64, W=128, seed=42):
     return inputs, flows, mobiles, cams, inst
 
 
+def save_split(name, arrays, part, moved_prefixes):
+    """Keeps each file under 1 MB: the arrays named with `moved_prefixes` go to `part`.npz (tests/golden_util.PARTS)."""
+    moved = {k: v for k, v in arrays.items() if k.startswith(moved_prefixes)}
+    np.savez_compressed(os.path.join(OUT, name + ".npz"), **{k: v for k, v in arrays.items() if k not in moved})
+    np.savez_compressed(os.path.join(OUT, part + ".npz"), **moved)
+
+
 def run_reference(opt, batch, mode, photo, ssim_on, weights):
     inputs, flows, mobiles, cams, inst = batch
     f = {k: v.clone().requires_grad_(True) for k, v in flows.items()}
@@ -92,7 +99,7 @@ def main():
         store["cam_%s" % key((i,))] = v.numpy()
     for b, d in enumerate(inst):
         store["inst_%d" % b] = np.packbits(d["instances"].pred_masks.numpy(), axis=-1)
-    np.savez_compressed(os.path.join(OUT, "netinit_inputs.npz"), **store)
+    save_split("netinit_inputs", store, "netinit_inputs_nets", ("flow_", "mob_", "cam_", "inst_"))
     weights = ref.gauss_distance_weight(4, H, W)
     for mode, photo, ssim_on, dmin in MODES:
         opt = synthetic.default_opt(B, H, W, disable_min=dmin)
@@ -110,7 +117,10 @@ def main():
                 rec["warps_" + key((i,))] = out["warps"][(i, 0)].detach().numpy()
             if photo:
                 rec["valids_" + key((i,))] = np.packbits(out["valids"][(i, 0)][:, :1].numpy(), axis=-1)
-        np.savez_compressed(os.path.join(OUT, "netinit_%s.npz" % mode), **rec)
+        if mode == "T":
+            save_split("netinit_T", rec, "netinit_T_warps", ("warps_",))
+        else:
+            np.savez_compressed(os.path.join(OUT, "netinit_%s.npz" % mode), **rec)
         print("netinit", mode, {k: float(v) for k, v in rec.items() if k.startswith("loss_")})
 
     # ---- stress: BASELINE configs[0] shape (B=4, 192x640); scalars + strided gradient samples

@@ -11,6 +11,16 @@ SCALES = [0, 1, 2, 3]
 NETINIT_MODES = {"SN": (True, True, False), "T": (True, True, False), "TG": (True, True, False),
                  "DC": (False, False, False), "DS": (False, False, True)}
 STRESS_MODES = {"SN": (True, True, False), "T": (True, True, False), "TG": (True, True, False), "DC": (False, False, False)}
+# fixtures stored in more than one file (each file stays under 1 MB): name -> its further parts
+PARTS = {"netinit_inputs": ["netinit_inputs_nets"], "netinit_T": ["netinit_T_warps"]}
+
+
+class Fixture(dict):
+    """The arrays of one fixture, gathered from all its files; `.files` lists the names like np.load's result."""
+
+    @property
+    def files(self):
+        return list(self)
 
 
 def key(k):
@@ -18,7 +28,7 @@ def key(k):
 
 
 def load_netinit_batch():
-    z = np.load(os.path.join(GOLD, "netinit_inputs.npz"))
+    z = load_outputs("netinit_inputs")
     B, H, W = 2, 64, 128
     inputs, flows, mobiles, cams = {}, {}, {}, {}
     for i in (0, -1, 1):
@@ -39,7 +49,11 @@ def load_netinit_batch():
 
 
 def load_outputs(name):
-    return np.load(os.path.join(GOLD, name + ".npz"))
+    z = Fixture()
+    for part in [name] + PARTS.get(name, []):
+        with np.load(os.path.join(GOLD, part + ".npz")) as f:
+            z.update((k, f[k]) for k in f.files)
+    return z
 
 
 def check_against_golden(z, got, photo, fwd_tol, grad_tol, full=True, check_maps=True, map_tol=None):
