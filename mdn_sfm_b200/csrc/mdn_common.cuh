@@ -14,29 +14,6 @@
 #include <cuda/ptx>
 #define MDN_DYN_SMEM(name) extern __shared__ __align__(128) float name[]
 #define MDN_LAUNCH(kernel, grid, block, smem, stream, ...) kernel<<<grid, block, smem, stream>>>(__VA_ARGS__)
-// Programmatic dependent launch: the grid may be scheduled while the previous kernel of the stream drains; the kernel
-// calls pdl_wait() before it touches global memory, so only its launch latency overlaps.  MDN_PDL (environment) is a
-// bit mask of the launches that carry the attribute: 1 source repack, 2 fused tile kernel, 4 finish, 8 scale_grads.
-// Default 0: measured on B200 (bench.py, graph replay) the attribute made the step slower, not faster.
-#include <stdlib.h>
-#include <utility>
-namespace mdn {
-inline int pdl_mask() {
-  static const int m = [] { const char* e = getenv("MDN_PDL"); return e ? atoi(e) : 0; }();
-  return m;
-}
-template <class... KArgs, class... Args>
-inline void launch_pdl(int which, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = (pdl_mask() & which) ? 1 : 0;
-  cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
-}
-}  // namespace mdn
-#define MDN_LAUNCH_PDL(which, kernel, grid, block, smem, stream, ...) ::mdn::launch_pdl(which, kernel, grid, block, smem, stream, __VA_ARGS__)
 #endif
 
 #include <stdint.h>
@@ -44,13 +21,6 @@ inline void launch_pdl(int which, void (*kernel)(KArgs...), dim3 grid, dim3 bloc
 #define MDN_DEV __device__ __forceinline__
 
 namespace mdn {
-
-// Waits for the previous kernel of the stream (no-op unless launched with MDN_LAUNCH_PDL)
-MDN_DEV void pdl_wait() {
-#ifndef MDN_EMU
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-#endif
-}
 
 // ---------------------------------------------------------------------------------------------------
 // Epipolar distance, loss_utils.py:64-67 with p1 = (x, y, 1), p2 = (u, v, 1) (loss_functions.py:120-122).

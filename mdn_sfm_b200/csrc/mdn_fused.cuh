@@ -74,9 +74,8 @@ template <bool B> struct BoolTag { static constexpr bool value = B; };
 
 // PAD: grid_sample padding mode of the flow warp (0 zeros = what the reference's callers pass, 1 border, 2 reflection)
 template <bool PHOTO, bool MAPS, int PAD = 0>
-__global__ void __launch_bounds__(FT, MDN_FUSED_MIN_CTAS) fused_tile_kernel(const __grid_constant__ KParams P) {
+__global__ void __launch_bounds__(FT, FUSED_MIN_CTAS) fused_tile_kernel(const __grid_constant__ KParams P) {
   MDN_DYN_SMEM(smem_raw);
-  pdl_wait();
   const int tid = threadIdx.x;
   const int t = tid & 31, g = tid >> 5;    // column pair, row group (= warp)
   if (blockIdx.x == 0 && tid == 0) *P.ticket = 0u;   // finish_kernel's completion ticket (it runs after this grid)
@@ -526,20 +525,12 @@ __global__ void __launch_bounds__(FT, MDN_FUSED_MIN_CTAS) fused_tile_kernel(cons
       // tiles that lie fully inside an even-width image (the common case): the own pairs are real, 8-byte aligned
       // pixels -- no reflection / slot arithmetic, one LDG.64 per flow plane, next row's flow loaded a row ahead
       const bool tile_full = weven & (x0 + TW <= w) & (y0 + TH <= h);
-#ifdef MDN_ABLATE_P1
-      const int it0 = N_IT;
-#else
       const int it0 = tile_full ? PR : 0;
-#endif
       Slot cur;
       // the first slot of the rolled loop (on a full tile: this thread's halo-ring slot) is prepared BEFORE the own rows, so that its
       // flow loads fly while the own rows are gathered (-1 % per step; the slot's geometry costs ten registers across the own rows)
       prep(it0, cur);
-#ifdef MDN_ABLATE_P1
-      if (false) {
-#else
       if (tile_full) {
-#endif
         unsigned o = (unsigned)(py0 * w + px0);
         float2 fxn = ldg2(flx + o), fyn = ldg2(fly + o);
         const float2 xs = make_float2((float)px0, (float)px1);
@@ -653,11 +644,7 @@ __global__ void __launch_bounds__(FT, MDN_FUSED_MIN_CTAS) fused_tile_kernel(cons
 #pragma unroll 1
       for (int c = 0; c < 3; ++c) {
         // -- P2: SSIM windows of channel c, 2 columns x WPR rows per patch
-#ifdef MDN_ABLATE_P2
-        if (false) {
-#else
         if (use_ssim) {
-#endif
 #pragma unroll 1
           for (int patch = tid; patch < NPATCH; patch += FT) {
             const int rg = patch / NCP, cp = patch - rg * NCP;
@@ -704,9 +691,7 @@ __global__ void __launch_bounds__(FT, MDN_FUSED_MIN_CTAS) fused_tile_kernel(cons
           }
           __syncthreads();
         }
-#ifndef MDN_ABLATE_P3
         if (border) p3(c, BoolTag<true>()); else p3(c, BoolTag<false>());
-#endif
         if (use_ssim) __syncthreads();   // Q (and, after the last channel, W) is rewritten next
       }
     }
@@ -765,13 +750,8 @@ __global__ void __launch_bounds__(FT, MDN_FUSED_MIN_CTAS) fused_tile_kernel(cons
       Row rows[PR];
 #pragma unroll
       for (int k = 0; k < PR; ++k) fetch(k, rows[k]);
-#ifdef MDN_ABLATE_P4
-#pragma unroll 1
-      for (int k = 0; k < 0; ++k) {
-#else
 #pragma unroll
       for (int k = 0; k < PR; ++k) {
-#endif
         const Row& cur = rows[k];
         const int y = py0 + k;
         // (w-1)/2 [grid_sample] * 2 [2g-1] / (w-1) [/= w-1] * sx [scale factor]
@@ -852,13 +832,9 @@ __global__ void __launch_bounds__(FT, MDN_FUSED_MIN_CTAS) fused_tile_kernel(cons
       for (int k = 0; k < PAIR_SLOTS; ++k) acc[k] += accp[k].x + accp[k].y;
     }
     flush_acc<PAIR_SLOTS>(acc, sm.red, pair * PAIR_SLOTS);
-#ifndef MDN_ABLATE_TAIL
     if (need_mask && own) tail(pair);
-#endif
   }
-#ifndef MDN_ABLATE_TAIL
   if (need_mask && !own) tail(0);
-#endif
 
   __syncthreads();
   for (int k = tid; k < NSLOT; k += FT) {

@@ -22,6 +22,7 @@
 #include <algorithm>
 #include <atomic>
 #include <stdio.h>
+#include <stdlib.h>
 #include <string.h>
 
 namespace mdn {
@@ -29,13 +30,11 @@ namespace mdn {
 // ----------------------------------------------------------------------------------------------- geometry
 constexpr int NTHREADS = 256;                         // block size of the small standalone kernels
 constexpr int PACK_PX = 4;                            // pixels per thread of ref_pack_kernel
-// fused kernel: TW x TH tile, one thread per 2-column x 4-row patch of pixels
+// fused kernel: TW x TH tile, one thread per 2-column x PR-row patch of pixels
 constexpr int TW = 64, TH = 16;
-#ifndef MDN_PATCH_ROWS
-#define MDN_PATCH_ROWS 2      // measured: 2 rows (256 threads / CTA) beats 4 rows (128 threads) at every shape tried
-#endif
-constexpr int PR = MDN_PATCH_ROWS;                           // rows of the per-thread pixel patch (2 or 4)
-static_assert((PR == 2 || PR == 4) && TH % PR == 0, "patch rows");
+// measured: 2 rows (256 threads / CTA) beats 4 rows (128 threads) at every shape tried
+constexpr int PR = 2;                                        // rows of the per-thread pixel patch
+static_assert(PR % 2 == 0 && TH % PR == 0, "patch rows (the SSIM adjoint gather takes them in pairs)");
 constexpr int FT = (TW / 2) * (TH / PR), FWARPS = FT / 32;   // lane = column pair, warp = row group
 static_assert(TW == 64, "one warp spans the tile width: 32 lanes x 2 columns");
 // halo-2 planes (target / warped image / mobile maps): rows y0-2 .. y0+TH+1, columns x0-2 .. x0+TW+1 (W2 = TW + 4 of
@@ -47,16 +46,11 @@ constexpr int W2 = TW + 4, S2 = TW + 8, R2H = TH + 4, OFF2 = 2, R2P = S2 * R2H;
 static_assert((R2P * 4) % 128 == 0 && S2 >= OFF2 + W2, "TMA box geometry");
 // halo-1 planes (SSIM adjoint coefficients): window rows y0-1 .. y0+TH, columns x0-1 .. x0+TW
 constexpr int S1 = TW + 4, R1H = TH + 2, R1P = S1 * R1H;
-#ifndef MDN_WPR
-#define MDN_WPR 3
-#endif
-constexpr int WPR = MDN_WPR;                                // window rows per SSIM patch (2 columns x WPR rows)
+constexpr int WPR = 3;                                      // window rows per SSIM patch (2 columns x WPR rows)
 static_assert((TH + 2) % WPR == 0, "SSIM patches tile the halo-1 region exactly");
 constexpr int NCP = (TW + 2) / 2, NPATCH = NCP * ((TH + 2) / WPR);
 constexpr int RING = W2 * R2H - TW * TH;              // halo slots of the halo-2 region
-#ifndef MDN_FUSED_MIN_CTAS
-#define MDN_FUSED_MIN_CTAS 2  // 128 registers / thread, no spills; the larger L1 carve-out of 2 CTAs / SM helps the gather
-#endif
+constexpr int FUSED_MIN_CTAS = 2;  // 128 registers / thread, no spills; the larger L1 carve-out of 2 CTAs / SM helps the gather
 
 // partial-sum slots per tile
 constexpr int PAIR_SLOTS = 16;   // epi, nt, ce, l1, ssim, gF[9], pad, pad
@@ -398,7 +392,6 @@ MDN_DEV void ref_pack_block(const KParams& P, const int bid) {
 // sharing a grid lets them overlap instead of running back to back (SN / DS / DC with the photometric term: -15 us per step).
 __global__ void __launch_bounds__(NTHREADS) ref_pack_kernel(const __grid_constant__ KParams P, unsigned long long* keys, const int n_pack,
                                                             const int n_sn, const int ratio, const int sn_chunks) {
-  pdl_wait();
   const int bid = blockIdx.x;
   if (n_sn == 0) { ref_pack_block(P, bid); return; }
   // the two kinds of blocks INTERLEAVED (`ratio` repack blocks, then one SN block, ...): blocks are dispatched in index
@@ -439,7 +432,6 @@ __global__ void __launch_bounds__(FIN_ROWS * NSLOT) finish_kernel(const __grid_c
   __shared__ float tots4[MDN_MAX_SCALES][NSLOT];
   __shared__ float pose_terms[MDN_MAX_SCALES][MDN_MAX_PAIRS][9];
   __shared__ bool is_last;
-  pdl_wait();
   const int b = blockIdx.x;
   const int slot = threadIdx.x % NSLOT, row = threadIdx.x / NSLOT;
   const bool grads = (P.flags & MDN_OPT_GRADS) != 0;
@@ -624,7 +616,6 @@ struct GradList {
 __global__ void __launch_bounds__(NTHREADS) scale_grads_kernel(const __grid_constant__ GradList L, const float* g, float* applied,
                                                                unsigned* ticket) {
   __shared__ bool is_last;
-  pdl_wait();
   const float gv = __ldg(g), ap = *applied;
   if (gv == ap) return;                      // loss.backward() with the implicit upstream gradient of 1: nothing to do
   const float ratio = gv / ap;
@@ -1078,7 +1069,7 @@ static int launch_fused(const MdnLossDesc* d, float* loss_out, void* workspace, 
   const int n_sn = sn_pass ? sn_chunks * (int)nkeys : 0;
   const int ratio = n_sn ? (n_pack + n_sn - 1) / n_sn : 0;            // repack blocks per SN block (0: SN blocks only)
   const int n_pre = n_sn ? std::max(n_sn, ratio ? (n_pack + ratio - 1) / ratio : 0) * (ratio + 1) : n_pack;
-  if (n_pre > 0) MDN_LAUNCH_PDL(1, ref_pack_kernel, dim3(n_pre), dim3(NTHREADS), 0, stream, K, keys, n_pack, n_sn, ratio, sn_chunks);
+  if (n_pre > 0) MDN_LAUNCH(ref_pack_kernel, dim3(n_pre), dim3(NTHREADS), 0, stream, K, keys, n_pack, n_sn, ratio, sn_chunks);
   // DS / DC: the instance masks may still be in flight on another stream (their preparation overlaps the pre-pass above);
   // the launches that read them wait for the caller's event here
   if (d->inst_ready && cudaStreamWaitEvent(stream, (cudaEvent_t)d->inst_ready, 0) != cudaSuccess) return fail(MDN_ERR_CUDA, "cudaStreamWaitEvent failed");
@@ -1090,22 +1081,18 @@ static int launch_fused(const MdnLossDesc* d, float* loss_out, void* workspace, 
       const MdnScale& S = d->scale[s];
       maps |= S.post_map[p] || S.ori_map[p] || S.warped[p] || S.diff[p] || S.valid[p] || S.ssim_map[p];
     }
-#ifndef MDN_PREFETCH_WAVES_X2
-#define MDN_PREFETCH_WAVES_X2 2      // prefetch distance in half waves (tuning macro; 2 = one wave)
-#endif
-  K.prefetch_distance = MDN_FUSED_MIN_CTAS * 148 * MDN_PREFETCH_WAVES_X2 / 2;   // one wave of resident CTAs (148 SMs on B200)
+  K.prefetch_distance = FUSED_MIN_CTAS * 148;   // one wave of resident CTAs (148 SMs on B200)
 #ifndef MDN_EMU
   {
     // TMA descriptors for the input tiles (target image, mobile maps): one box copy per plane instead of ~400 cp.async
-    // with their index arithmetic.  MDN_NO_TMA=1 (environment) keeps the cp.async staging.
+    // with their index arithmetic.  A scale keeps the cp.async staging where its row pitch is not a multiple of 16 bytes
+    // or a descriptor could not be encoded (no cuTensorMapEncodeTiled from the driver).
     typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
     static EncodeFn encode = [] {
       void* fn = nullptr;
       cudaDriverEntryPointQueryResult q;
-      const char* off = getenv("MDN_NO_TMA");
-      if (off && off[0] == '1') return (EncodeFn) nullptr;
       if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) != cudaSuccess) fn = nullptr;
       return (EncodeFn)fn;
     }();
@@ -1139,6 +1126,13 @@ static int launch_fused(const MdnLossDesc* d, float* loss_out, void* workspace, 
 #endif
   if (ev) cudaEventRecord(ev[1], stream);
   const dim3 grid(K.n_tiles), block(FT);
+  // the instantiations, indexed [pad][photo][maps].  PAD is the padding_mode of the flow warp (0 zeros, 1 border,
+  // 2 reflection); only the photometric term warps, so without it every pad index holds the zeros-padding kernels.
+  using FusedFn = void (*)(KParams);
+  static const FusedFn fused_kernels[3][2][2] = {
+      {{fused_tile_kernel<false, false>, fused_tile_kernel<false, true>}, {fused_tile_kernel<true, false>, fused_tile_kernel<true, true>}},
+      {{fused_tile_kernel<false, false>, fused_tile_kernel<false, true>}, {fused_tile_kernel<true, false, 1>, fused_tile_kernel<true, true, 1>}},
+      {{fused_tile_kernel<false, false>, fused_tile_kernel<false, true>}, {fused_tile_kernel<true, false, 2>, fused_tile_kernel<true, true, 2>}}};
   // > 48 KB of dynamic shared memory needs the opt-in attribute, per device (idempotent; set once per device).  The bit is
   // published only after every attribute call succeeded, with an atomic OR: concurrent first calls from two host threads
   // may both set the attributes (harmless) but never see a half-initialised device.
@@ -1150,14 +1144,11 @@ static int launch_fused(const MdnLossDesc* d, float* loss_out, void* workspace, 
   const unsigned long long dev_bit = 1ull << (dev_index & 63);
   if (!(smem_opt_in_devices.load(std::memory_order_acquire) & dev_bit)) {
     const int bytes = (int)(fused_smem_floats(true) * sizeof(float));
-    cudaError_t a = cudaFuncSetAttribute(fused_tile_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-    if (a == cudaSuccess) a = cudaFuncSetAttribute(fused_tile_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-    if (a == cudaSuccess) a = cudaFuncSetAttribute(fused_tile_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-    if (a == cudaSuccess) a = cudaFuncSetAttribute(fused_tile_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-    if (a == cudaSuccess) a = cudaFuncSetAttribute(fused_tile_kernel<true, true, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-    if (a == cudaSuccess) a = cudaFuncSetAttribute(fused_tile_kernel<true, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-    if (a == cudaSuccess) a = cudaFuncSetAttribute(fused_tile_kernel<true, true, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
-    if (a == cudaSuccess) a = cudaFuncSetAttribute(fused_tile_kernel<true, false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    cudaError_t a = cudaSuccess;
+    for (const auto& by_photo : fused_kernels)
+      for (const auto& by_maps : by_photo)
+        for (const FusedFn kfn : by_maps)
+          if (a == cudaSuccess) a = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
     if (a != cudaSuccess) {
       cudaGetLastError();
       snprintf(g_err, sizeof(g_err), "the fused kernel needs %d bytes of opt-in shared memory per block on device %d: %s", bytes, dev_index,
@@ -1166,18 +1157,11 @@ static int launch_fused(const MdnLossDesc* d, float* loss_out, void* workspace, 
     }
     smem_opt_in_devices.fetch_or(dev_bit, std::memory_order_release);
   }
-  // padding_mode of the flow warp other than zeros: its own instantiations (the zeros-padding kernels are untouched)
   const int pad = (d->flags & MDN_OPT_PAD_BORDER) ? 1 : ((d->flags & MDN_OPT_PAD_REFLECTION) ? 2 : 0);
-  if (photo && pad == 1 && maps) { auto kfn = fused_tile_kernel<true, true, 1>; MDN_LAUNCH_PDL(2, kfn, grid, block, smem, stream, K); }
-  else if (photo && pad == 1) { auto kfn = fused_tile_kernel<true, false, 1>; MDN_LAUNCH_PDL(2, kfn, grid, block, smem, stream, K); }
-  else if (photo && pad == 2 && maps) { auto kfn = fused_tile_kernel<true, true, 2>; MDN_LAUNCH_PDL(2, kfn, grid, block, smem, stream, K); }
-  else if (photo && pad == 2) { auto kfn = fused_tile_kernel<true, false, 2>; MDN_LAUNCH_PDL(2, kfn, grid, block, smem, stream, K); }
-  else if (photo && maps) { auto kfn = fused_tile_kernel<true, true>; MDN_LAUNCH_PDL(2, kfn, grid, block, smem, stream, K); }
-  else if (photo) { auto kfn = fused_tile_kernel<true, false>; MDN_LAUNCH_PDL(2, kfn, grid, block, smem, stream, K); }
-  else if (maps) { auto kfn = fused_tile_kernel<false, true>; MDN_LAUNCH_PDL(2, kfn, grid, block, smem, stream, K); }
-  else { auto kfn = fused_tile_kernel<false, false>; MDN_LAUNCH_PDL(2, kfn, grid, block, smem, stream, K); }
+  const FusedFn kfn = fused_kernels[pad][photo][maps];
+  MDN_LAUNCH(kfn, grid, block, smem, stream, K);
   if (ev) cudaEventRecord(ev[2], stream);
-  MDN_LAUNCH_PDL(4, finish_kernel, dim3(d->batch), dim3(FIN_ROWS * NSLOT), 0, stream, Q);
+  MDN_LAUNCH(finish_kernel, dim3(d->batch), dim3(FIN_ROWS * NSLOT), 0, stream, Q);
   if (ev) cudaEventRecord(ev[3], stream);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return fail(MDN_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
@@ -1226,7 +1210,7 @@ extern "C" MDN_API int mdn_loss_scale_grads(const MdnLossDesc* d, const float* g
   }
   if (L.n == 0) return MDN_OK;
   // applied[1] (MDN_OUT_APPLIED + 1) is the completion ticket, zeroed by mdn_loss_fused
-  MDN_LAUNCH_PDL(8, scale_grads_kernel, dim3(296), dim3(NTHREADS), 0, stream, L, g, applied, reinterpret_cast<unsigned*>(applied + 1));
+  MDN_LAUNCH(scale_grads_kernel, dim3(296), dim3(NTHREADS), 0, stream, L, g, applied, reinterpret_cast<unsigned*>(applied + 1));
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return fail(MDN_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
   return MDN_OK;

@@ -1,7 +1,7 @@
 """Kernel-variant timing: python scripts/kbench.py lib1.so [lib2.so ...] [--shape HxW] [--batch B] [--mode T] [--iters N]
 
 Times Loss.forward (= fundamental prologue + mdn_loss_fused) with CUDA events over 4 rotating input sets for each
-library build given on the command line (e.g. builds of mdn_loss.cu with different -D tuning macros).  Experiment
+library build given on the command line (any builds of libmdn_loss.so, for example of two commits).  Experiment
 tooling: bench.py is the number of record.
 """
 import os

@@ -20,7 +20,7 @@ inputs, flows, mobiles, cams, inst = synthetic.make_batch(B, H, W, scales=scales
                                                           with_instances=mode in ("DS", "DC"))
 flows = {k: v.requires_grad_(True) for k, v in flows.items()}
 mobiles = {k: v.requires_grad_(True) for k, v in mobiles.items()}
-if "--lib" in sys.argv:   # a tuning build (scripts/build_variant.sh) instead of the in-tree library
+if "--lib" in sys.argv:   # another build of libmdn_loss.so instead of the in-tree library
     from mdn_sfm_b200 import _cabi
     _cabi._lib = _cabi.Library(os.path.abspath(sys.argv[sys.argv.index("--lib") + 1]))
 loss = Loss(opt, no_ssim=False, mode=mode, photometric=True)

@@ -146,7 +146,6 @@ inline uint32_t exchange(uint32_t v, int src_tid) {
 #define MDN_DYN_SMEM(name) float* name = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(mdn_emu::st().smem.data()) + 63) & ~uintptr_t(63))
 #define MDN_LAUNCH(kernel, grid, block, smem, stream, ...) \
   mdn_emu::launch(grid, block, smem, [=]() { kernel(__VA_ARGS__); })
-#define MDN_LAUNCH_PDL(which, kernel, grid, block, smem, stream, ...) MDN_LAUNCH(kernel, grid, block, smem, stream, __VA_ARGS__)
 
 static inline void __syncthreads() { mdn_emu::yield_to_scheduler(); }
 static inline void __threadfence() {}
