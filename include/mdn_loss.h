@@ -258,6 +258,12 @@ MDN_API int mdn_ssim_bwd(const float* x, const float* y, const float* g_out, flo
  */
 MDN_API int mdn_instance_mask_union(const uint8_t* const* masks, const int32_t* counts, uint8_t* out, int32_t batch,
                                     int64_t hw, void* stream);
+/* The same union as mdn_instance_mask_union, but `masks` (batch device pointers) and `counts` (batch int32) are DEVICE
+ * arrays, read by the kernel when it runs.  Captured into a CUDA graph, it follows whatever the tables hold at replay time.
+ * The tables and the masks they point to must stay valid until the work has run.  counts[b] <= 0 gives an all-zero sample.
+ * batch <= 65535; one launch. */
+MDN_API int mdn_instance_mask_union_table(const uint8_t* const* masks, const int32_t* counts, uint8_t* out,
+                                          int32_t batch, int64_t hw, void* stream);
 MDN_API int mdn_instance_mask_resize(const uint8_t* src, int32_t batch, int32_t in_h, int32_t in_w, uint8_t* const* dst,
                                      const int32_t* out_h, const int32_t* out_w, int32_t n_out, void* workspace,
                                      size_t workspace_bytes, void* stream);

@@ -53,7 +53,7 @@ EXPORTS = ("mdn_version", "mdn_last_error_string", "mdn_loss_workspace_bytes", "
            "mdn_fundamental_fwd", "mdn_fundamental_bwd",
            "mdn_epipolar_points_fwd", "mdn_epipolar_points_bwd", "mdn_epipolar_points_workspace_bytes",
            "mdn_flow_warp_fwd", "mdn_flow_warp_bwd", "mdn_ssim_fwd", "mdn_ssim_bwd", "mdn_binary_image",
-           "mdn_instance_mask_union", "mdn_instance_mask_resize", "mdn_instance_mask_resize_workspace_bytes", "mdn_image_pyramid", "mdn_image_pyramid_packed", "mdn_normalize_u8")
+           "mdn_instance_mask_union", "mdn_instance_mask_union_table", "mdn_instance_mask_resize", "mdn_instance_mask_resize_workspace_bytes", "mdn_image_pyramid", "mdn_image_pyramid_packed", "mdn_normalize_u8")
 
 
 class Library:
@@ -85,6 +85,7 @@ class Library:
             "mdn_ssim_bwd": (C.c_int, [_P, _P, _P, _P, _P, i32, i32, i32, _P]),
             "mdn_binary_image": (C.c_int, [_P, _P, i64, f32, _P]),
             "mdn_instance_mask_union": (C.c_int, [C.POINTER(_P), C.POINTER(i32), _P, i32, i64, _P]),
+            "mdn_instance_mask_union_table": (C.c_int, [_P, _P, _P, i32, i64, _P]),
             "mdn_instance_mask_resize": (C.c_int, [_P, i32, i32, i32, C.POINTER(_P), C.POINTER(i32), C.POINTER(i32), i32, _P, sz, _P]),
             "mdn_image_pyramid": (C.c_int, [_P, i32, i32, i32, C.POINTER(_P), C.POINTER(i32), C.POINTER(i32), i32, _P, sz, _P]),
             "mdn_normalize_u8": (C.c_int, [_P, _P, i32, i32, i32, C.POINTER(f32), C.POINTER(f32), _P]),

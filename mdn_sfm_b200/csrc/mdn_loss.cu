@@ -11,7 +11,7 @@
 //   finish_kernel        deterministic second stage, one block per sample: tile sums -> d/dF, SN arg-max fix-up, pose
 //                        adjoint; last block -> loss scalars
 //   scale_grads_kernel   backward for an upstream gradient != 1 (exits immediately when it is 1)
-//   instance_union / instance_resize_{weights,h,v}_kernel   DS / DC instance masks and fp32 image pyramids (torchvision
+//   instance_union{,_table} / instance_resize_{weights,h,v}_kernel   DS / DC instance masks and fp32 image pyramids (torchvision
 //                        antialiased Resize replayed)
 //   small standalone kernels for the individually exported reference functions
 //
@@ -1341,6 +1341,16 @@ extern "C" MDN_API int mdn_instance_mask_union(const uint8_t* const* masks, cons
     }
     MDN_LAUNCH(instance_union_kernel, dim3(blocks_for(hw, 296), nb), dim3(NTHREADS), 0, (cudaStream_t)stream, A, out + (long long)b0 * hw, (long long)hw);
   }
+  cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? MDN_OK : fail(MDN_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
+}
+
+extern "C" MDN_API int mdn_instance_mask_union_table(const uint8_t* const* masks, const int32_t* counts, uint8_t* out,
+                                                     int32_t batch, int64_t hw, void* stream) {
+  if (!masks || !counts || !out) return fail(MDN_ERR_NULL_POINTER, "masks / counts / out is NULL");
+  if (batch < 1 || batch > 65535 || hw < 1) return fail(MDN_ERR_BAD_SHAPE, "batch / hw out of range");
+  MDN_LAUNCH(instance_union_table_kernel, dim3(blocks_for(hw, 296), batch), dim3(NTHREADS), 0, (cudaStream_t)stream, masks,
+             (const int*)counts, out, (long long)hw);
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? MDN_OK : fail(MDN_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
 }

@@ -1,6 +1,6 @@
 // mdn_resize.cuh -- instance-mask union and the antialiased-bilinear resize (torchvision Resize / ATen
 // _upsample_bilinear2d_aa replayed) for {0,1} masks and fp32 image pyramids.  Included by mdn_loss.cu INSIDE namespace mdn.
-// Entry points: mdn_instance_mask_union / _resize, mdn_image_pyramid / _packed (include/mdn_loss.h).
+// Entry points: mdn_instance_mask_union / _union_table / _resize, mdn_image_pyramid / _packed (include/mdn_loss.h).
 
 // get_batch_instance_mask (loss_utils.py:102-124): union of the N boolean instance masks of a sample.
 constexpr int UNION_CHUNK = 32;   // samples per launch (pointer table passed by value)
@@ -9,11 +9,9 @@ struct UnionArgs {
   int count[UNION_CHUNK];
 };
 
-__global__ void __launch_bounds__(NTHREADS) instance_union_kernel(const __grid_constant__ UnionArgs A, uint8_t* __restrict__ out, long long hw) {
-  const int b = blockIdx.y;
-  const uint8_t* src = A.masks[b];
-  const int n = A.count[b];
-  uint8_t* dst = out + (long long)b * hw;
+// One sample's union, spread over the blocks of grid.x: `n` planes of `hw` bytes at `src` -> `hw` bytes {0,1} at `dst`
+// (n <= 0: all zero).  Four, two or one pixel per thread, as `hw` and the alignment of `src` / `dst` allow.
+MDN_DEV void instance_union_sample(const uint8_t* src, int n, uint8_t* dst, long long hw) {
   const bool wide = (hw & 3) == 0 && ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & 3) == 0;
   if (wide) {   // four pixels per thread
     const long long n4 = hw >> 2;
@@ -54,6 +52,20 @@ __global__ void __launch_bounds__(NTHREADS) instance_union_kernel(const __grid_c
     for (int k = 0; k < n; ++k) v |= __ldg(src + (long long)k * hw + i);   // sum(pred_masks, 0) != 0
     dst[i] = v ? 1 : 0;
   }
+}
+
+__global__ void __launch_bounds__(NTHREADS) instance_union_kernel(const __grid_constant__ UnionArgs A, uint8_t* __restrict__ out, long long hw) {
+  const int b = blockIdx.y;
+  instance_union_sample(A.masks[b], A.count[b], out + (long long)b * hw, hw);
+}
+
+// The same union with the (pointer, count) table in device memory, read when the kernel runs: a CUDA graph that
+// captured this launch follows whatever the table holds at replay time.  One launch, grid.y = batch.
+__global__ void __launch_bounds__(NTHREADS) instance_union_table_kernel(const uint8_t* const* __restrict__ masks,
+                                                                        const int* __restrict__ counts,
+                                                                        uint8_t* __restrict__ out, long long hw) {
+  const int b = blockIdx.y;
+  instance_union_sample(masks[b], counts[b], out + (long long)b * hw, hw);
 }
 
 // torchvision Resize (bilinear, antialias, align_corners=False) of a {0,1} mask followed by round-to-nearest-even, as

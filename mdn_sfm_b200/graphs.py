@@ -15,7 +15,8 @@ class GraphedLossStep:
 
     flows / mobiles / cams whose tensors require grad must be LEAF tensors; after ``replay()`` their ``.grad`` holds the
     gradient of the step (the same graph-owned buffers every time).  ``instances`` (DS / DC) are prepared inside the
-    capture, so their mask tensors must be static too."""
+    capture: pass a ``loss_utils.InstanceMaskTable`` and ``load`` each batch into it before ``replay()`` (the union kernel
+    reads the table when it runs); a list / bare ``Instances`` is replayed with the masks it was captured with."""
 
     def __init__(self, loss, inputs, frame_ids, flows, mobiles, instances, scales, cams, warmup=3):
         self.loss_module = loss
@@ -89,7 +90,10 @@ class GraphedLoss:
     autograd node passes the replay's gradients on to the nets.  The (non-differentiable) ``inputs`` are copied only when
     they are not the static tensors themselves: a loader that writes each batch into ``static_inputs`` pays no copy.
     ``unit_upstream`` (set by TrainStep around ``loss.backward()``): the upstream gradient is known to be 1, skip the rescale.
-    Detectron2 instances (DS / DC) change shape per batch and are not supported here -- use the eager ``Loss`` for them."""
+    Detectron2 instances (DS / DC), as a list of ``{"instances": obj}`` or one bare ``Instances``, may hold a different
+    number of masks every batch: each call loads their pointers and counts into a device table
+    (``loss_utils.InstanceMaskTable``) that the captured union kernel reads at replay.  Their form, the batch size and the
+    mask size are part of the capture key; a new mask size captures again."""
 
     def __init__(self, loss):
         self.loss_module = loss
@@ -101,15 +105,25 @@ class GraphedLoss:
     def _pose_tensors(c):
         return (c.axisangle, c.translation) if hasattr(c, "axisangle") else (c,)
 
-    def _signature(self, inputs, frame_ids, flows, mobiles, scales, cams):
-        sig = [tuple(frame_ids), tuple(scales)]
+    @staticmethod
+    def _instance_form(instances, batch):
+        """(form, B, H, W, device) of the Detectron2 masks of a batch: everything a capture depends on but the counts."""
+        if instances is None:
+            return None
+        from .loss_utils import _pred_masks
+        m = _pred_masks(instances)[0]
+        return ("list" if isinstance(instances, list) else "bare", batch, int(m.shape[-2]), int(m.shape[-1]), m.device)
+
+    def _signature(self, inputs, frame_ids, flows, mobiles, scales, cams, inst_form):
+        sig = [tuple(frame_ids), tuple(scales), inst_form]
         for d in (inputs, flows, mobiles):
             sig.append(tuple((k, tuple(v.shape), v.requires_grad) for k, v in d.items()))
         sig.append(tuple((k, type(c).__name__, tuple(tuple(t.shape) + (t.requires_grad,) for t in self._pose_tensors(c))) for k, c in cams.items()))
         return tuple(sig)
 
-    def _capture(self, inputs, frame_ids, flows, mobiles, scales, cams):
+    def _capture(self, inputs, frame_ids, flows, mobiles, instances, inst_form, scales, cams):
         from .layers import PoseParameters
+        from .loss_utils import InstanceMaskTable
         own = lambda t: t.detach().clone().requires_grad_(t.requires_grad)
         self.static_inputs = {k: v.detach().clone() for k, v in inputs.items()}
         s_flows = {k: own(v) for k, v in flows.items()}
@@ -117,7 +131,11 @@ class GraphedLoss:
         s_cams = {k: (PoseParameters(own(c.axisangle), own(c.translation)) if hasattr(c, "axisangle") else own(c)) for k, c in cams.items()}
         self.static_args = (s_flows, s_mobiles, s_cams)
         self.static_diff = [t for t in self._diff_list(s_flows, s_mobiles, s_cams)]
-        self.step = GraphedLossStep(self.loss_module, self.static_inputs, frame_ids, s_flows, s_mobiles, None, scales, s_cams)
+        self.table = None
+        if inst_form is not None:      # the capture's warm-up steps already read the first batch's masks
+            _, B, H, W, dev = inst_form
+            self.table = InstanceMaskTable(B, H, W, dev).load(instances)
+        self.step = GraphedLossStep(self.loss_module, self.static_inputs, frame_ids, s_flows, s_mobiles, self.table, scales, s_cams)
 
     def _diff_list(self, flows, mobiles, cams):
         out = [t for d in (flows, mobiles) for t in d.values() if t.requires_grad]
@@ -130,12 +148,13 @@ class GraphedLoss:
             torch._foreach_copy_([s for s in self.static_diff], [t.detach() for t in tensors])
 
     def __call__(self, inputs, frame_ids, flows, mobiles, instances, scales, cams):
-        if instances is not None:
-            raise NotImplementedError("GraphedLoss: Detectron2 instances change shape per batch; use the eager Loss for DS / DC")
-        key = self._signature(inputs, frame_ids, flows, mobiles, scales, cams)
+        inst_form = self._instance_form(instances, next(iter(flows.values())).shape[0])
+        key = self._signature(inputs, frame_ids, flows, mobiles, scales, cams, inst_form)
         if self.step is None or key != self.key:
-            self._capture(inputs, list(frame_ids), flows, mobiles, list(scales), cams)
+            self._capture(inputs, list(frame_ids), flows, mobiles, instances, inst_form, list(scales), cams)
             self.key = key
+        elif instances is not None:
+            self.table.load(instances)      # this batch's masks: written ahead of the replay in stream order
         with torch.no_grad():      # the batch itself: copied only when the caller did not write it into static_inputs
             src = [(self.static_inputs[k], v) for k, v in inputs.items() if v.data_ptr() != self.static_inputs[k].data_ptr()]
             if src:

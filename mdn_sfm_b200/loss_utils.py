@@ -14,7 +14,7 @@ from .ops import EpipolarPointsFn, FlowWarpFn, _c
 
 __all__ = ["inverse_warp", "get_epipolar_new", "detectron2_similarity_loss", "post_pro_epipolar_weighted",
            "post_process_epipolar_1", "get_batch_instance_mask", "post_process_epipolar_2", "create_coords",
-           "smooth_loss", "derivable_consistency_loss", "compute_quantiles"]
+           "smooth_loss", "derivable_consistency_loss", "compute_quantiles", "InstanceMaskTable"]
 
 
 def _arith_flag(arith):
@@ -59,6 +59,63 @@ def _pred_masks(instances_info):
     return [instances_info.pred_masks]
 
 
+class InstanceMaskTable:
+    """A batch's Detectron2 instance masks as a DEVICE table -- B mask pointers (int64) and B instance counts (int32) -- for
+    `mdn_instance_mask_union_table`, which reads the table when its kernel runs.  A CUDA graph that captured the union
+    therefore follows each new batch: `load` the batch, then replay.  Pass the table where `instances_info` goes
+    (`instance_masks_u8`, `Loss.forward`).
+
+    `load` writes the table in the current stream's order (a non-blocking copy from pinned host memory), so work queued
+    after it on that stream sees the new batch, and work queued before it the old one.  The table keeps the mask tensors
+    alive until the next `load`."""
+
+    def __init__(self, batch, height, width, device):
+        if batch < 1 or height < 1 or width < 1:
+            raise ValueError("InstanceMaskTable needs batch, height and width >= 1")
+        self.batch, self.height, self.width = int(batch), int(height), int(width)
+        self.device = torch.device(device)
+        if self.device.type == "cuda" and self.device.index is None:
+            self.device = torch.device("cuda", torch.cuda.current_device())
+        # one buffer, one copy per load: B pointers, then B counts (int32, two per int64 slot)
+        self._words = self.batch + (self.batch + 1) // 2
+        self._table = torch.zeros(self._words, dtype=torch.int64, device=self.device)
+        self.ptrs = self._table[:self.batch]
+        self.counts = self._table[self.batch:].view(torch.int32)[:self.batch]
+        self.masks = []
+
+    def _check(self, m):
+        if m.dtype != torch.bool and m.dtype != torch.uint8:
+            raise TypeError("mdn_sfm_b200: pred_masks must be bool or uint8 (got %s)" % m.dtype)
+        if m.device != self.device:
+            raise ValueError("mdn_sfm_b200: pred_masks on %s, the instance table on %s" % (m.device, self.device))
+        if m.dim() != 3 or tuple(m.shape[1:]) != (self.height, self.width):
+            raise ValueError("mdn_sfm_b200: pred_masks must be (N, %d, %d) (got %s)" % (self.height, self.width, tuple(m.shape)))
+        if not m.is_contiguous():
+            raise ValueError("mdn_sfm_b200: pred_masks must be contiguous")
+        return _cabi.check_tensor(m.view(torch.uint8) if m.dtype == torch.bool else m, dtype=torch.uint8, what="pred_masks")
+
+    def load(self, instances_info):
+        """Points the table at this batch's masks: a list of B {"instances": obj} dicts, or one bare `Instances` whose masks
+        every sample of the batch uses (the reference's (1,3,H,W) mask broadcast over the batch)."""
+        masks = [self._check(m) for m in _pred_masks(instances_info)]
+        if isinstance(instances_info, list) and len(masks) != self.batch:
+            raise ValueError("instances_info holds %d samples, the instance table %d" % (len(masks), self.batch))
+        per_sample = masks if isinstance(instances_info, list) else masks * self.batch
+        host = torch.empty(self._words, dtype=torch.int64, pin_memory=self.device.type == "cuda")
+        h = host.numpy()
+        h[:self.batch] = [m.data_ptr() for m in per_sample]
+        h[self.batch:].view("int32")[:self.batch] = [m.shape[0] for m in per_sample]
+        if self.device.type == "cuda":
+            self._table.copy_(host, non_blocking=True)      # the caching host allocator holds `host` until the copy has run
+            stream = torch.cuda.current_stream(self.device)
+            for m in masks:
+                m.record_stream(stream)
+        else:
+            self._table.copy_(host)
+        self.masks = masks
+        return self
+
+
 def instance_masks_u8(instances_info, sizes, device, library=None, batch=None):
     """One-channel uint8 {0,1} instance masks at every size in `sizes` (a list of (h, w)), from ONE pass over the
     Detectron2 masks: `get_batch_instance_mask` (loss_utils.py:102-124: union of the instances of each sample) and the
@@ -66,24 +123,33 @@ def instance_masks_u8(instances_info, sizes, device, library=None, batch=None):
     back to integers) run as two kernels -- `mdn_instance_mask_union`, `mdn_instance_mask_resize` -- instead of the
     reference's per-(frame, scale) int64 (B,3,375,1242) tensors.  The three channels upstream carries are identical;
     one is kept.  -> list of (B, h, w) uint8 tensors.  `batch`: the batch size of the maps the masks will meet; a single
-    bare `Instances` (trainer.py:494, evaluate_mix.py:63) then broadcasts over it like the reference's (1,3,H,W) mask."""
+    bare `Instances` (trainer.py:494, evaluate_mix.py:63) then broadcasts over it like the reference's (1,3,H,W) mask.
+    `instances_info` may also be an InstanceMaskTable (then `device` is the table's): the union reads it on the device."""
     import ctypes as C
     library = library or _cabi.lib()
-    masks = []
-    for m in _pred_masks(instances_info):
-        m = m.to(device)
-        if m.dtype != torch.bool and m.dtype != torch.uint8:
-            m = m != 0
-        m = m.contiguous()
-        masks.append(_cabi.check_tensor(m.view(torch.uint8) if m.dtype == torch.bool else m, dtype=torch.uint8, what="pred_masks"))
-    B = len(masks)
-    H, W = masks[0].shape[-2:]
-    if any(tuple(m.shape[-2:]) != (H, W) for m in masks):
-        raise ValueError("instance masks of one batch must share their size")
-    union = torch.empty((B, H, W), dtype=torch.uint8, device=masks[0].device)
-    stream = _cabi.stream_ptr(union)
-    counts = (C.c_int32 * B)(*[int(m.shape[0]) if m.dim() == 3 else 1 for m in masks])
-    library.call("mdn_instance_mask_union", _cabi.ptr_array(masks), counts, union.data_ptr(), B, H * W, stream, dev=union)
+    if isinstance(instances_info, InstanceMaskTable):     # the union reads the device table: capturable in a CUDA graph
+        T = instances_info
+        B, H, W = T.batch, T.height, T.width
+        union = torch.empty((B, H, W), dtype=torch.uint8, device=T.device)
+        stream = _cabi.stream_ptr(union)
+        library.call("mdn_instance_mask_union_table", T.ptrs.data_ptr(), T.counts.data_ptr(), union.data_ptr(), B, H * W,
+                     stream, dev=union)
+    else:
+        masks = []
+        for m in _pred_masks(instances_info):
+            m = m.to(device)
+            if m.dtype != torch.bool and m.dtype != torch.uint8:
+                m = m != 0
+            m = m.contiguous()
+            masks.append(_cabi.check_tensor(m.view(torch.uint8) if m.dtype == torch.bool else m, dtype=torch.uint8, what="pred_masks"))
+        B = len(masks)
+        H, W = masks[0].shape[-2:]
+        if any(tuple(m.shape[-2:]) != (H, W) for m in masks):
+            raise ValueError("instance masks of one batch must share their size")
+        union = torch.empty((B, H, W), dtype=torch.uint8, device=masks[0].device)
+        stream = _cabi.stream_ptr(union)
+        counts = (C.c_int32 * B)(*[int(m.shape[0]) if m.dim() == 3 else 1 for m in masks])
+        library.call("mdn_instance_mask_union", _cabi.ptr_array(masks), counts, union.data_ptr(), B, H * W, stream, dev=union)
     outs = [torch.empty((B, int(h), int(w)), dtype=torch.uint8, device=union.device) for h, w in sizes]
     for k0 in range(0, len(outs), _cabi.MAX_SCALES):
         chunk = outs[k0:k0 + _cabi.MAX_SCALES]

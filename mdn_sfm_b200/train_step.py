@@ -138,10 +138,11 @@ class TrainStep:
 
     def __init__(self, opt, nets=None, loss_module=None, device="cuda", lr=1e-4, clip_grad=1.0,
                  fine_tune_flow_motion=False, mode="TG", photometric=True, graph_loss=True, pose_params=True):
-        """graph_loss: run the CUDA loss path as one CUDA-graph replay per step (graphs.GraphedLoss; batches without
-        Detectron2 instances).  pose_params: hand PoseNet's (axisangle, translation) to the loss as parameters so that the
-        fused call also runs transformation_from_parameters and its adjoint (layers.PoseParameters).  Both apply to the
-        default CUDA loss only; a caller-supplied `loss_module` gets the reference's (B,4,4) matrices, eagerly."""
+        """graph_loss: run the CUDA loss path as one CUDA-graph replay per step (graphs.GraphedLoss; in DS / DC mode the
+        batches' new Detectron2 instances replay the same graph).  pose_params: hand PoseNet's (axisangle, translation) to
+        the loss as parameters so that the fused call also runs transformation_from_parameters and its adjoint
+        (layers.PoseParameters).  Both apply to the default CUDA loss only; a caller-supplied `loss_module` gets the
+        reference's (B,4,4) matrices, eagerly."""
         self.opt, self.device = opt, torch.device(device)
         self.nets = (nets or StandInNets()).to(self.device)
         self.fine_tune = fine_tune_flow_motion
@@ -186,8 +187,7 @@ class TrainStep:
             flows.update(flow)
             mobiles.update(self.mobile_decoder(feats, axisangle, translation, frame_id=i))
             cams[i] = PoseParameters(axisangle, translation) if self.pose_params else transformation_from_parameters(axisangle, translation)
-        loss = self.loss if (instances is None or self.eager_loss is None) else self.eager_loss     # (DS / DC batches: eager launches)
-        outputs, losses = loss(inputs, ids, flows, mobiles, instances, list(o.scales), cams)
+        outputs, losses = self.loss(inputs, ids, flows, mobiles, instances, list(o.scales), cams)
         return flows, mobiles, cams, outputs, losses
 
     def step(self, inputs, instances=None):
