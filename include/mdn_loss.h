@@ -303,6 +303,27 @@ MDN_API int mdn_normalize_u8(const uint8_t* src, float* dst, int32_t batch, int3
 /* binary_image (utils.py:100-103): out = x >= threshold ? 1 : 0 */
 MDN_API int mdn_binary_image(const float* x, float* out, int64_t n, float threshold, void* stream);
 
+/*
+ * Evaluation of mobile masks for a whole threshold sweep in one pass over the maps: the confusion counts of
+ * binary_image(pred, thr) (utils.py:100-103) against moving-object masks, for every image and threshold.
+ *
+ * pred (batch, hw) fp32 mobile probabilities; gt (batch, hw) uint8, non-zero = moving (get_batch_instance_mask's != 0);
+ * thresholds: n_thr fp32 values, 1 <= n_thr <= 1024.  A pixel is predicted moving at threshold t iff pred >= t in fp32:
+ * a prediction equal to a threshold is moving at it, NaN is never moving, -0.0 >= 0.0.
+ * counts (batch, n_thr, 4) int64 = [TP, FP, FN, TN] per image and threshold, exact; each row sums to hw.
+ *
+ * The thresholds must be strictly increasing and free of NaN (+-inf allowed): that is the CALLER's precondition, not
+ * checked here.  Other thresholds give wrong counts, never an access outside the arrays.
+ * workspace: mdn_mask_confusion_workspace_bytes(batch, n_thr) bytes (per-sample histograms; 0 on bad arguments).
+ * Three operations on `stream`: a memset of the workspace, the counting kernel, the finish kernel.
+ * Errors: NULL argument; batch outside 1..65535, hw outside 1..2^31-1 or n_thr outside 1..1024 (MDN_ERR_BAD_SHAPE);
+ * a pointer that is not 16-byte aligned; a workspace that is too small.
+ */
+MDN_API size_t mdn_mask_confusion_workspace_bytes(int32_t batch, int32_t n_thr);
+MDN_API int mdn_mask_confusion(const float* pred, const uint8_t* gt, const float* thresholds, int32_t n_thr,
+                               int64_t* counts, int32_t batch, int64_t hw, void* workspace, size_t workspace_bytes,
+                               void* stream);
+
 #ifdef __cplusplus
 }
 #endif

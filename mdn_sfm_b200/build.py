@@ -14,7 +14,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 SRC = os.path.join(HERE, "csrc", "mdn_loss.cu")
-DEPS = [SRC, os.path.join(HERE, "csrc", "mdn_common.cuh"), os.path.join(HERE, "csrc", "mdn_fused.cuh"), os.path.join(HERE, "csrc", "mdn_resize.cuh"), os.path.join(ROOT, "include", "mdn_loss.h")]
+DEPS = [SRC, os.path.join(HERE, "csrc", "mdn_common.cuh"), os.path.join(HERE, "csrc", "mdn_fused.cuh"), os.path.join(HERE, "csrc", "mdn_resize.cuh"), os.path.join(HERE, "csrc", "mdn_metrics.cuh"), os.path.join(ROOT, "include", "mdn_loss.h")]
 OUT_DIR = os.path.join(HERE, "_lib")
 OUT = os.path.join(OUT_DIR, "libmdn_loss.so")
 

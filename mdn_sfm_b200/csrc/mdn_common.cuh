@@ -8,6 +8,7 @@
 
 #ifdef MDN_EMU
 #include "cuda_emu.h"
+#include "cuda_emu_match.h"   // __match_any_sync, __popc, __ffs (tests/emu)
 #else
 #include <cuda.h>
 #include <cuda_runtime.h>

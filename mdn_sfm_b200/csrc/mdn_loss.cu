@@ -13,6 +13,7 @@
 //   scale_grads_kernel   backward for an upstream gradient != 1 (exits immediately when it is 1)
 //   instance_union{,_table} / instance_resize_{weights,h,v}_kernel   DS / DC instance masks and fp32 image pyramids (torchvision
 //                        antialiased Resize replayed)
+//   mask_confusion{,_finish}_kernel   evaluation: [TP, FP, FN, TN] of binary_image(mobile, thr) for a threshold sweep
 //   small standalone kernels for the individually exported reference functions
 //
 // All of it is bandwidth/latency-bound stencil + gather work: no tensor cores by design.
@@ -841,6 +842,9 @@ __global__ void __launch_bounds__(NTHREADS) ssim_bwd_kernel(const float* __restr
 // ----------------------------------------------------------------------------------------------- instance masks, pyramids
 #include "mdn_resize.cuh"
 
+// ----------------------------------------------------------------------------------------------- mask evaluation
+#include "mdn_metrics.cuh"
+
 __global__ void __launch_bounds__(NTHREADS) binary_image_kernel(const float* __restrict__ x, float* __restrict__ out, long long n, float thr) {
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
     out[i] = (x[i] >= thr) ? 1.f : 0.f;
@@ -1496,5 +1500,41 @@ extern "C" MDN_API int mdn_binary_image(const float* x, float* out, int64_t n, f
   if (n < 1) return MDN_OK;
   MDN_LAUNCH(binary_image_kernel, dim3(blocks_for(n)), dim3(NTHREADS), 0, (cudaStream_t)stream, x, out, (long long)n, threshold);
   cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? MDN_OK : fail(MDN_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
+}
+
+extern "C" MDN_API size_t mdn_mask_confusion_workspace_bytes(int32_t batch, int32_t n_thr) {
+  if (batch < 1 || batch > 65535 || n_thr < 1 || n_thr > CONF_MAX_THR) {
+    fail(MDN_ERR_BAD_SHAPE, "batch / n_thr out of range");
+    return 0;
+  }
+  return (size_t)batch * 2 * (size_t)(n_thr + 1) * sizeof(unsigned);
+}
+
+extern "C" MDN_API int mdn_mask_confusion(const float* pred, const uint8_t* gt, const float* thresholds, int32_t n_thr,
+                                          int64_t* counts, int32_t batch, int64_t hw, void* workspace,
+                                          size_t workspace_bytes, void* stream) {
+  if (!pred || !gt || !thresholds || !counts || !workspace)
+    return fail(MDN_ERR_NULL_POINTER, "pred / gt / thresholds / counts / workspace is NULL");
+  if (batch < 1 || batch > 65535 || hw < 1 || hw > 2147483647ll || n_thr < 1 || n_thr > CONF_MAX_THR)
+    return fail(MDN_ERR_BAD_SHAPE, "batch / hw / n_thr out of range");
+  if (!aligned16(pred) || !aligned16(gt) || !aligned16(thresholds) || !aligned16(counts) || !aligned16(workspace))
+    return fail(MDN_ERR_MISALIGNED, "%s is not 16-byte aligned", "pred / gt / thresholds / counts / workspace");
+  const size_t need = mdn_mask_confusion_workspace_bytes(batch, n_thr);
+  if (workspace_bytes < need) return fail(MDN_ERR_WORKSPACE, "workspace too small");
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaError_t e = cudaMemsetAsync(workspace, 0, need, st);
+  if (e != cudaSuccess) return fail(MDN_ERR_CUDA, "cudaMemsetAsync failed: %s", cudaGetErrorString(e));
+  int top = 1;
+  while (2 * top <= n_thr) top *= 2;
+  // enough pixels per block that the flush of its 2 (K + 1) bins stays small next to its counting; at most about
+  // 8 blocks per SM over the batch
+  const long long per_block = std::max<long long>(CONF_THREADS * 16, 8ll * 2 * (n_thr + 1));
+  const long long bx = std::max<long long>(1, std::min<long long>((hw + per_block - 1) / per_block, (148 * 8 + batch - 1) / batch));
+  MDN_LAUNCH(mask_confusion_kernel, dim3((unsigned)bx, batch), dim3(CONF_THREADS), 0, st, pred, gt, thresholds, (int)n_thr,
+             top, (unsigned*)workspace, (long long)hw);
+  MDN_LAUNCH(mask_confusion_finish_kernel, dim3(batch), dim3(CONF_THREADS), 0, st, (const unsigned*)workspace, (int)n_thr,
+             (long long*)counts);
+  e = cudaGetLastError();
   return e == cudaSuccess ? MDN_OK : fail(MDN_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
 }
