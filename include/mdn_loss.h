@@ -324,6 +324,42 @@ MDN_API int mdn_mask_confusion(const float* pred, const uint8_t* gt, const float
                                int64_t* counts, int32_t batch, int64_t hw, void* workspace, size_t workspace_bytes,
                                void* stream);
 
+/*
+ * Evaluation of optical flow in one pass over the ground truth: end-point error (EPE) and KITTI Fl outliers per image and
+ * region, from the network's flow at its own resolution.
+ *
+ * flow (batch, 2, h, w) fp32, the prediction at any resolution; gt_flow (batch, 2, H, W) fp32 in pixels of H x W;
+ * gt_valid (batch, H, W) uint8, non-zero = valid; region (batch, H, W) uint8 labels, or NULL = every pixel in region 0
+ * (then n_regions must be 1).  counts (batch, n_regions, 2) int64 = [valid, outliers]; epe_sum (batch, n_regions) fp64.
+ *
+ * Per ground-truth pixel (y, x) of sample b, every operation fp32 and rounded on its own (no contraction):
+ *   1. source row (ATen upsample_bilinear2d, align_corners=False, no scale_factor): ry = float(h) / float(H),
+ *      sy = ry * (float(y) + 0.5f) - 0.5f, 0 if below 0; y0 = (int)sy, dy = (y0 < h-1), ly1 = sy - y0, ly0 = 1 - ly1;
+ *      the column likewise with w and W
+ *   2. per channel c: f_c = ly0*(lx0*F[y0][x0] + lx1*F[y0][x0+dx]) + ly1*(lx0*F[y0+dy][x0] + lx1*F[y0+dy][x0+dx]) in
+ *      that order (at h = H, w = W this is the input, except that 0 * a non-finite neighbour gives NaN as in ATen)
+ *   3. u = f_0 * scale_x, v = f_1 * scale_y
+ *   4. e = sqrt((u-gu)*(u-gu) + (v-gv)*(v-gv)), m = sqrt(gu*gu + gv*gv)
+ *   5. outlier = e > abs_thr && e / m > rel_thr (the KITTI devkit's Fl test: abs_thr 3, rel_thr 0.05); m = 0 gives inf
+ *      or NaN and the comparison treats it as IEEE does; a NaN e is never an outlier but does reach epe_sum
+ *   6. the pixel counts iff gt_valid != 0 and its label r < n_regions (so 255 can mean "ignore"): it adds 1 to
+ *      valid[b][r], outlier to outliers[b][r] and (double)e to epe_sum[b][r]
+ *   7. an uncounted pixel's ground truth reaches no sum, whatever it holds (KITTI stores 0 there, other loaders NaN)
+ * The fp64 sums are fixed trees over a grid that depends on the shapes only: bit-identical run to run and on any device.
+ *
+ * workspace: mdn_flow_errors_workspace_bytes(...) bytes (per-block partials; 0 on bad arguments).  Two kernels on
+ * `stream`, no allocation, no synchronisation, no copy.
+ * Errors: a NULL required pointer, or a NULL region with n_regions > 1 (MDN_ERR_NULL_POINTER); batch outside 1..65535,
+ * a size < 1, h*w or H*W above 2^31-1, n_regions outside 1..8, a non-finite scale or threshold or a negative threshold
+ * (MDN_ERR_BAD_SHAPE); a pointer that is not 16-byte aligned; a workspace that is too small.
+ */
+MDN_API size_t mdn_flow_errors_workspace_bytes(int32_t batch, int32_t height, int32_t width, int32_t gt_height,
+                                               int32_t gt_width, int32_t n_regions);
+MDN_API int mdn_flow_errors(const float* flow, int32_t height, int32_t width, float scale_x, float scale_y,
+                            const float* gt_flow, const uint8_t* gt_valid, const uint8_t* region, int32_t n_regions,
+                            int32_t gt_height, int32_t gt_width, int32_t batch, float abs_thr, float rel_thr,
+                            int64_t* counts, double* epe_sum, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

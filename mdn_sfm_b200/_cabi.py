@@ -54,7 +54,7 @@ EXPORTS = ("mdn_version", "mdn_last_error_string", "mdn_loss_workspace_bytes", "
            "mdn_epipolar_points_fwd", "mdn_epipolar_points_bwd", "mdn_epipolar_points_workspace_bytes",
            "mdn_flow_warp_fwd", "mdn_flow_warp_bwd", "mdn_ssim_fwd", "mdn_ssim_bwd", "mdn_binary_image",
            "mdn_instance_mask_union", "mdn_instance_mask_union_table", "mdn_instance_mask_resize", "mdn_instance_mask_resize_workspace_bytes", "mdn_image_pyramid", "mdn_image_pyramid_packed", "mdn_normalize_u8",
-           "mdn_mask_confusion", "mdn_mask_confusion_workspace_bytes")
+           "mdn_mask_confusion", "mdn_mask_confusion_workspace_bytes", "mdn_flow_errors", "mdn_flow_errors_workspace_bytes")
 
 
 class Library:
@@ -94,6 +94,8 @@ class Library:
             "mdn_instance_mask_resize_workspace_bytes": (sz, [i32, i32, i32, C.POINTER(i32), C.POINTER(i32), i32]),
             "mdn_mask_confusion": (C.c_int, [_P, _P, _P, i32, _P, i32, i64, _P, sz, _P]),
             "mdn_mask_confusion_workspace_bytes": (sz, [i32, i32]),
+            "mdn_flow_errors": (C.c_int, [_P, i32, i32, f32, f32, _P, _P, _P, i32, i32, i32, i32, f32, f32, _P, _P, _P, sz, _P]),
+            "mdn_flow_errors_workspace_bytes": (sz, [i32, i32, i32, i32, i32, i32]),
         }
         for name, (res, args) in sig.items():
             fn = getattr(d, name)

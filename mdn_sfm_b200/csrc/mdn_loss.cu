@@ -14,6 +14,7 @@
 //   instance_union{,_table} / instance_resize_{weights,h,v}_kernel   DS / DC instance masks and fp32 image pyramids (torchvision
 //                        antialiased Resize replayed)
 //   mask_confusion{,_finish}_kernel   evaluation: [TP, FP, FN, TN] of binary_image(mobile, thr) for a threshold sweep
+//   flow_errors{,_finish}_kernel   evaluation: end-point error and KITTI Fl outliers per image and region
 //   small standalone kernels for the individually exported reference functions
 //
 // All of it is bandwidth/latency-bound stencil + gather work: no tensor cores by design.
@@ -22,6 +23,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <cmath>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -845,6 +847,9 @@ __global__ void __launch_bounds__(NTHREADS) ssim_bwd_kernel(const float* __restr
 // ----------------------------------------------------------------------------------------------- mask evaluation
 #include "mdn_metrics.cuh"
 
+// ----------------------------------------------------------------------------------------------- flow evaluation
+#include "mdn_flow_eval.cuh"
+
 __global__ void __launch_bounds__(NTHREADS) binary_image_kernel(const float* __restrict__ x, float* __restrict__ out, long long n, float thr) {
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
     out[i] = (x[i] >= thr) ? 1.f : 0.f;
@@ -1536,5 +1541,73 @@ extern "C" MDN_API int mdn_mask_confusion(const float* pred, const uint8_t* gt, 
   MDN_LAUNCH(mask_confusion_finish_kernel, dim3(batch), dim3(CONF_THREADS), 0, st, (const unsigned*)workspace, (int)n_thr,
              (long long*)counts);
   e = cudaGetLastError();
+  return e == cudaSuccess ? MDN_OK : fail(MDN_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
+}
+
+// Blocks per sample of flow_errors_kernel: a function of the ground-truth size alone, never of the device.
+static int flow_errors_blocks(long long gt_hw) {
+  const long long quads = (gt_hw + 3) / 4, per_block = (long long)FE_THREADS * FE_QUADS_PER_THREAD;
+  return (int)std::max<long long>(1, std::min<long long>((quads + per_block - 1) / per_block, FE_MAX_BLOCKS));
+}
+
+static bool flow_errors_shape_ok(int32_t batch, int32_t height, int32_t width, int32_t gt_height, int32_t gt_width,
+                                 int32_t n_regions) {
+  return batch >= 1 && batch <= 65535 && height >= 1 && width >= 1 && gt_height >= 1 && gt_width >= 1 &&
+         (long long)height * width <= 2147483647ll && (long long)gt_height * gt_width <= 2147483647ll &&
+         n_regions >= 1 && n_regions <= FE_MAX_REGIONS;
+}
+
+extern "C" MDN_API size_t mdn_flow_errors_workspace_bytes(int32_t batch, int32_t height, int32_t width,
+                                                          int32_t gt_height, int32_t gt_width, int32_t n_regions) {
+  if (!flow_errors_shape_ok(batch, height, width, gt_height, gt_width, n_regions)) {
+    fail(MDN_ERR_BAD_SHAPE, "batch / sizes / n_regions out of range");
+    return 0;
+  }
+  const size_t parts = (size_t)batch * flow_errors_blocks((long long)gt_height * gt_width) * n_regions;
+  return parts * (sizeof(double) + 2 * sizeof(long long));
+}
+
+template <int RT>
+static void flow_errors_launch(const FlowArgs& a, int batch, long long* counts, double* epe_sum, cudaStream_t st) {
+  MDN_LAUNCH(flow_errors_kernel<RT>, dim3(a.nblk, batch), dim3(FE_THREADS), 0, st, a);
+  MDN_LAUNCH(flow_errors_finish_kernel<RT>, dim3(batch), dim3(FE_THREADS), 0, st, (const double*)a.part_sum,
+             (const long long*)a.part_cnt, a.nblk, a.R, counts, epe_sum);
+}
+
+extern "C" MDN_API int mdn_flow_errors(const float* flow, int32_t height, int32_t width, float scale_x, float scale_y,
+                                       const float* gt_flow, const uint8_t* gt_valid, const uint8_t* region,
+                                       int32_t n_regions, int32_t gt_height, int32_t gt_width, int32_t batch,
+                                       float abs_thr, float rel_thr, int64_t* counts, double* epe_sum, void* workspace,
+                                       size_t workspace_bytes, void* stream) {
+  if (!flow || !gt_flow || !gt_valid || !counts || !epe_sum || !workspace)
+    return fail(MDN_ERR_NULL_POINTER, "flow / gt_flow / gt_valid / counts / epe_sum / workspace is NULL");
+  if (!region && n_regions > 1) return fail(MDN_ERR_NULL_POINTER, "region is NULL with n_regions > 1");
+  if (!flow_errors_shape_ok(batch, height, width, gt_height, gt_width, n_regions))
+    return fail(MDN_ERR_BAD_SHAPE, "batch / sizes / n_regions out of range");
+  if (!std::isfinite(scale_x) || !std::isfinite(scale_y) || !std::isfinite(abs_thr) || !std::isfinite(rel_thr) ||
+      abs_thr < 0.f || rel_thr < 0.f)
+    return fail(MDN_ERR_BAD_SHAPE, "scale / threshold out of range (non-finite or a negative threshold)");
+  if (!aligned16(flow) || !aligned16(gt_flow) || !aligned16(gt_valid) || (region && !aligned16(region)) ||
+      !aligned16(counts) || !aligned16(epe_sum) || !aligned16(workspace))
+    return fail(MDN_ERR_MISALIGNED, "%s is not 16-byte aligned",
+                "flow / gt_flow / gt_valid / region / counts / epe_sum / workspace");
+  const size_t need = mdn_flow_errors_workspace_bytes(batch, height, width, gt_height, gt_width, n_regions);
+  if (workspace_bytes < need) return fail(MDN_ERR_WORKSPACE, "workspace too small");
+  FlowArgs a;
+  a.flow = flow; a.gt = gt_flow; a.valid = gt_valid; a.region = region;
+  a.nblk = flow_errors_blocks((long long)gt_height * gt_width);
+  a.part_sum = (double*)workspace;
+  a.part_cnt = (long long*)(a.part_sum + (size_t)batch * a.nblk * n_regions);
+  a.h = height; a.w = width; a.H = gt_height; a.W = gt_width; a.R = n_regions;
+  a.ry = (float)height / (float)gt_height;     // ATen's area_pixel_compute_scale: input / output in fp32
+  a.rx = (float)width / (float)gt_width;
+  a.scale_x = scale_x; a.scale_y = scale_y; a.abs_thr = abs_thr; a.rel_thr = rel_thr;
+  cudaStream_t st = (cudaStream_t)stream;
+  long long* c = (long long*)counts;
+  if (n_regions == 1) flow_errors_launch<1>(a, batch, c, epe_sum, st);
+  else if (n_regions == 2) flow_errors_launch<2>(a, batch, c, epe_sum, st);
+  else if (n_regions <= 4) flow_errors_launch<4>(a, batch, c, epe_sum, st);
+  else flow_errors_launch<8>(a, batch, c, epe_sum, st);
+  cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? MDN_OK : fail(MDN_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
 }
