@@ -140,12 +140,6 @@ def check_tensor(t, dtype=torch.float32, what="tensor"):
     return t
 
 
-def on_device(t):
-    """Context manager that makes `t`'s CUDA device current (a no-op for host tensors: the emulated test build)."""
-    import contextlib
-    return torch.cuda.device(t.device) if t.is_cuda else contextlib.nullcontext()
-
-
 def stream_ptr(ref_tensor):
     return torch.cuda.current_stream(ref_tensor.device).cuda_stream if ref_tensor.is_cuda else 0
 

@@ -157,51 +157,6 @@ MDN_DEV void bilinear_deriv(const Bilin& b, float nw, float ne, float sw, float 
   ddy = b.ax0 * (sw - nw) + b.ax1 * (se - ne);
 }
 
-// Branch-free variant used by the fused kernel: corner offsets clamped into the plane, zeros padding applied by
-// multiplying the loaded values with 0/1 masks, so the 4 x C loads of a pixel can all be in flight together.
-struct Gather4 {
-  int o00, o01, o10, o11;       // element offsets of the nw, ne, sw, se corners inside one channel plane (always valid)
-  float m00, m01, m10, m11;     // 1 if that corner lies inside the image, else 0
-  float ax0, ax1, ay0, ay1;     // (x0+1-ix), (ix-x0), (y0+1-iy), (iy-y0)
-};
-
-MDN_DEV Gather4 gather_setup(float ix, float iy, int h, int w) {
-  Gather4 g;
-  const float x0f = floorf(ix), y0f = floorf(iy);
-  g.ax0 = (x0f + 1.f) - ix; g.ax1 = ix - x0f;
-  g.ay0 = (y0f + 1.f) - iy; g.ay1 = iy - y0f;
-  int x0 = min(max(__float2int_rd(ix), -2), w), y0 = min(max(__float2int_rd(iy), -2), h);   // NaN -> 0, huge -> outside
-  const int x1 = x0 + 1, y1 = y0 + 1;
-  const bool bx0 = (unsigned)x0 < (unsigned)w, bx1 = (unsigned)x1 < (unsigned)w;
-  const bool by0 = (unsigned)y0 < (unsigned)h, by1 = (unsigned)y1 < (unsigned)h;
-  const int cx0 = bx0 ? x0 : 0, cx1 = bx1 ? x1 : 0;
-  const int r0 = (by0 ? y0 : 0) * w, r1 = (by1 ? y1 : 0) * w;
-  g.o00 = r0 + cx0; g.o01 = r0 + cx1; g.o10 = r1 + cx0; g.o11 = r1 + cx1;
-  const float fx0 = bx0 ? 1.f : 0.f, fx1 = bx1 ? 1.f : 0.f, fy0 = by0 ? 1.f : 0.f, fy1 = by1 ? 1.f : 0.f;
-  g.m00 = fx0 * fy0; g.m01 = fx1 * fy0; g.m10 = fx0 * fy1; g.m11 = fx1 * fy1;
-  return g;
-}
-
-MDN_DEV void gather_fetch(const float* __restrict__ plane, const Gather4& g, float& nw, float& ne, float& sw, float& se) {
-  nw = __ldg(plane + g.o00) * g.m00;
-  ne = __ldg(plane + g.o01) * g.m01;
-  sw = __ldg(plane + g.o10) * g.m10;
-  se = __ldg(plane + g.o11) * g.m11;
-}
-
-MDN_DEV float gather_value(const Gather4& g, float nw, float ne, float sw, float se) {
-  float o = nw * (g.ax0 * g.ay0);
-  o += ne * (g.ax1 * g.ay0);
-  o += sw * (g.ax0 * g.ay1);
-  o += se * (g.ax1 * g.ay1);
-  return o;
-}
-
-MDN_DEV void gather_deriv(const Gather4& g, float nw, float ne, float sw, float se, float& ddx, float& ddy) {
-  ddx = g.ay0 * (ne - nw) + g.ay1 * (se - sw);
-  ddy = g.ax0 * (sw - nw) + g.ax1 * (se - ne);
-}
-
 // ---------------------------------------------------------------------------------------------------
 // Packed fp32x2 arithmetic (Blackwell FADD2 / FMUL2 / FFMA2: two IEEE-rn results per issue slot).  The FP32 pipe
 // does the same lane-operations per clock either way; what the packed forms save is ISSUE slots, which is what
@@ -239,88 +194,16 @@ MDN_DEV float2 ld2s(const float* p) { return *reinterpret_cast<const float2*>(p)
 MDN_DEV void st2s(float* p, float2 v) { *reinterpret_cast<float2*>(p) = v; }
 
 // ---------------------------------------------------------------------------------------------------
-// Two horizontally adjacent output pixels of the flow warp at once (packed fp32x2): the coordinate chain of
-// warp_coord() with the same roundings (2 g - 1 and (g + 1) / 2 * (n - 1) need one rounding each because the
-// doubling / halving is exact), the bilinear footprint with the zero padding folded into the FRACTIONS (a masked
-// fraction zeroes both the value weight and the derivative coefficient of its corners), values and
-// d(value)/d(ix, iy) of the three channels.  Corner addresses are clamped into the plane, so every load is legal
-// and the 24 loads of a pixel pair are in flight together.
-struct Gather2 {
-  float2 val[3];      // warped value, channel c   (x = first pixel, y = second)
-  float2 dx[3], dy[3];
-  bool valid_a, valid_b;
-};
-
-template <bool DERIV>
-MDN_DEV void gather_pair(const float* __restrict__ pl0, const float* __restrict__ pl1, const float* __restrict__ pl2, int h, int w,
-                         float2 xs, float2 ys, float2 fx, float2 fy, const WarpGeom& G, Gather2& out) {
-  const float2 one = splat2(1.f), neg1 = splat2(-1.f), two = splat2(2.f);
-  // NOTE: fx / fy must come from SCALAR multiplies: ptxas contracts mul.rn.f32x2 + add.rn.f32x2 into FFMA2 (it
-  // honours .rn only for scalar ops), which would move x + sx * f by an ulp and flip bilinear cells
-  const float2 px = add2(xs, fx), py = add2(ys, fy);
-  float2 gx, gy;
-  if (G.cuda_arith) { gx = mul2(px, splat2(G.inv_wm1)); gy = mul2(py, splat2(G.inv_hm1)); }
-  else {
-    gx = make_float2(__fdiv_rn(px.x, G.wm1), __fdiv_rn(px.y, G.wm1));
-    gy = make_float2(__fdiv_rn(py.x, G.hm1), __fdiv_rn(py.y, G.hm1));
-  }
-  gx = fma2(two, gx, neg1);                     // loss_utils.py:31
-  gy = fma2(two, gy, neg1);
-  out.valid_a = (fabsf(gx.x) <= 1.f) & (fabsf(gy.x) <= 1.f);
-  out.valid_b = (fabsf(gx.y) <= 1.f) & (fabsf(gy.y) <= 1.f);
-  const float2 ix = mul2(add2(gx, one), splat2(0.5f * G.wm1));   // grid_sample un-normalisation, align_corners=True
-  const float2 iy = mul2(add2(gy, one), splat2(0.5f * G.hm1));
-  const float2 x0f = make_float2(floorf(ix.x), floorf(ix.y)), y0f = make_float2(floorf(iy.x), floorf(iy.y));
-  float2 ax1 = fma2(x0f, neg1, ix), ax0 = fma2(ix, neg1, add2(x0f, one));
-  float2 ay1 = fma2(y0f, neg1, iy), ay0 = fma2(iy, neg1, add2(y0f, one));
-  unsigned o00[2], o01[2], o10[2], o11[2];
-  float mx0[2], mx1[2], my0[2], my1[2];
-#pragma unroll
-  for (int e = 0; e < 2; ++e) {
-    const int x0 = min(max(__float2int_rd(e ? ix.y : ix.x), -2), w), y0 = min(max(__float2int_rd(e ? iy.y : iy.x), -2), h);
-    const int x1 = x0 + 1, y1 = y0 + 1;
-    const bool bx0 = (unsigned)x0 < (unsigned)w, bx1 = (unsigned)x1 < (unsigned)w;
-    const bool by0 = (unsigned)y0 < (unsigned)h, by1 = (unsigned)y1 < (unsigned)h;
-    const unsigned cx0 = bx0 ? x0 : 0, cx1 = bx1 ? x1 : 0;
-    const unsigned r0 = (by0 ? y0 : 0) * w, r1 = (by1 ? y1 : 0) * w;
-    o00[e] = r0 + cx0; o01[e] = r0 + cx1; o10[e] = r1 + cx0; o11[e] = r1 + cx1;
-    mx0[e] = bx0 ? 1.f : 0.f; mx1[e] = bx1 ? 1.f : 0.f; my0[e] = by0 ? 1.f : 0.f; my1[e] = by1 ? 1.f : 0.f;
-  }
-  const float2 fx0 = make_float2(mx0[0], mx0[1]), fx1 = make_float2(mx1[0], mx1[1]);
-  const float2 fy0 = make_float2(my0[0], my0[1]), fy1 = make_float2(my1[0], my1[1]);
-  ax0 = mul2(ax0, fx0); ax1 = mul2(ax1, fx1); ay0 = mul2(ay0, fy0); ay1 = mul2(ay1, fy1);
-  const float2 w00 = mul2(ax0, ay0), w01 = mul2(ax1, ay0), w10 = mul2(ax0, ay1), w11 = mul2(ax1, ay1);
-  float2 cx00, cx01, cx10, cx11, cy00, cy01, cy10, cy11;
-  if (DERIV) {
-    const float2 nfx0 = mul2(fx0, neg1), nfy0 = mul2(fy0, neg1);
-    cx00 = mul2(ay0, nfx0); cx01 = mul2(ay0, fx1); cx10 = mul2(ay1, nfx0); cx11 = mul2(ay1, fx1);
-    cy00 = mul2(ax0, nfy0); cy01 = mul2(ax1, nfy0); cy10 = mul2(ax0, fy1); cy11 = mul2(ax1, fy1);
-  }
-  float2 v00[3], v01[3], v10[3], v11[3];
-#pragma unroll
-  for (int c = 0; c < 3; ++c) {
-    const float* pl = c == 0 ? pl0 : (c == 1 ? pl1 : pl2);
-    v00[c] = make_float2(__ldg(pl + o00[0]), __ldg(pl + o00[1]));
-    v01[c] = make_float2(__ldg(pl + o01[0]), __ldg(pl + o01[1]));
-    v10[c] = make_float2(__ldg(pl + o10[0]), __ldg(pl + o10[1]));
-    v11[c] = make_float2(__ldg(pl + o11[0]), __ldg(pl + o11[1]));
-  }
-#pragma unroll
-  for (int c = 0; c < 3; ++c) {
-    out.val[c] = fma2(v11[c], w11, fma2(v10[c], w10, fma2(v01[c], w01, mul2(v00[c], w00))));
-    if (DERIV) {
-      out.dx[c] = fma2(v11[c], cx11, fma2(v10[c], cx10, fma2(v01[c], cx01, mul2(v00[c], cx00))));
-      out.dy[c] = fma2(v11[c], cy11, fma2(v10[c], cy10, fma2(v01[c], cy01, mul2(v00[c], cy00))));
-    }
-  }
-}
-
-// The same for a source image REPACKED to one float4 (r, g, b, -) per pixel (ref_pack_kernel): the four corners of
-// a pixel are four 16-byte loads that bring all three channels at once -- a third of the load instructions and of
-// the L1 wavefronts / L2 sector requests of the planar form, which is what bounds the gather when neighbouring
-// pixels sample unrelated places.  Coordinates, fractions and masks are packed over the two PIXELS as above; the
-// interpolation is packed over the (r, g) CHANNELS of one pixel with the weight as the broadcast scalar operand,
-// b is scalar.  Output: per pixel e (0 / 1) value and derivatives of the three channels.
+// Two horizontally adjacent output pixels of the flow warp at once, from a source image REPACKED to one float4
+// (r, g, b, -) per pixel (ref_pack_kernel).  The coordinate chain is warp_coord()'s with the same roundings (2 g - 1
+// and (g + 1) / 2 * (n - 1) need one rounding each because the doubling / halving is exact).  Zero padding is folded
+// into the bilinear FRACTIONS: a masked fraction zeroes both the value weight and the derivative coefficient of its
+// corners.  Corner addresses are clamped into the image, so every load is legal and the loads of a pixel pair are in
+// flight together.  The four corners of a pixel are four 16-byte loads that bring all three channels at once -- a
+// third of the load instructions and of the L1 wavefronts / L2 sector requests of a planar gather, which is what
+// bounds the gather when neighbouring pixels sample unrelated places.  Coordinates, fractions and masks are packed
+// over the two PIXELS; the interpolation is packed over the (r, g) CHANNELS of one pixel with the weight as the
+// broadcast scalar operand, b is scalar.  Output: per pixel e (0 / 1) value and derivatives of the three channels.
 struct GatherPx {
   float v[3], dx[3], dy[3];
 };
@@ -331,7 +214,9 @@ template <bool DERIV, int PAD = PAD_ZEROS>
 MDN_DEV void gather_pair_packed(const float4* __restrict__ pk, int h, int w, float2 xs, float2 ys, float2 fx, float2 fy,
                                 const WarpGeom& G, GatherPx* out, bool& valid_a, bool& valid_b) {
   const float2 one = splat2(1.f), neg1 = splat2(-1.f), two = splat2(2.f);
-  const float2 px = add2(xs, fx), py = add2(ys, fy);     // fx / fy from SCALAR multiplies (see gather_pair)
+  // NOTE: fx / fy must come from SCALAR multiplies: ptxas contracts mul.rn.f32x2 + add.rn.f32x2 into FFMA2 (it
+  // honours .rn only for scalar ops), which would move x + sx * f by an ulp and flip bilinear cells
+  const float2 px = add2(xs, fx), py = add2(ys, fy);
   float2 gx, gy;
   if (G.cuda_arith) { gx = mul2(px, splat2(G.inv_wm1)); gy = mul2(py, splat2(G.inv_hm1)); }
   else {
@@ -414,13 +299,6 @@ struct SsimOut {
   float dmu_y, dY2, dXY;   // dz/d(mu_y) (total, incl. through sigma_y, sigma_xy), dz/dE[y^2], dz/dE[xy]; 0 outside the clamp gate
   float dmu_x, dX2;        // same for x (used by the standalone SSIM backward)
 };
-
-// s / 9 correctly rounded without the IEEE-division subroutine: one Newton step on q = s * rn(1/9) (Markstein)
-MDN_DEV float div9(float s) {
-  const float r9 = 0.111111111f;
-  float q = __fmul_rn(s, r9);
-  return __fmaf_rn(__fmaf_rn(-9.f, q, s), r9, q);
-}
 
 MDN_DEV SsimOut ssim_window(float sx, float sy, float sxx, float syy, float sxy, bool want_grad) {
   const float C1 = 0.0001f, C2 = 0.0009f;
@@ -548,7 +426,6 @@ MDN_DEV void cp_async_wait_all() {
 #endif
 }
 
-MDN_DEV float sigmoidf_(float x) { return 1.f / (1.f + expf(-x)); }
 MDN_DEV float signf_(float x) { return (x > 0.f) ? 1.f : ((x < 0.f) ? -1.f : 0.f); }
 // signf_(x) * v, bit for bit (v finite), in three instructions instead of five: the sign bit of x flips v; zero / NaN x give 0
 MDN_DEV float signmul(float x, float v) {

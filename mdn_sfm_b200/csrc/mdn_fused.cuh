@@ -18,7 +18,7 @@
 //   sFL [PR][2][FT]  thread-private float2 slots: the flow of the own pixels (P1 -> P4)
 // Per pair (with the poses given, nine threads first rebuild F = K^-T [t]x R K^-1 of the (pair, sample)):
 //   P1  one rolled loop over pixel PAIRS: the thread's PR own pairs, then its share of the halo ring.  flow ->
-//       sampling coordinates -> bilinear gather of the 3 source channels (gather_pair) -> sW; derivatives -> sD
+//       sampling coordinates -> bilinear gather of the 3 source channels (gather_pair_packed) -> sW; derivatives -> sD
 //   per channel c (rolled):
 //     P2  SSIM windows over the tile + 1-pixel halo in 2x3 patches: 3-tap row sums of (x, y, x^2, y^2, xy) for two
 //         columns from two LDS.64 per image row, a sliding column sum, two windows per packed evaluation
@@ -554,7 +554,7 @@ __global__ void __launch_bounds__(FT, FUSED_MIN_CTAS) fused_tile_kernel(const __
         else { nxt = cur; nxt.live = false; }
         if (!cur.live) break;
         const bool oka = (cur.ya | cur.xa) >= 0, okb = (cur.ya | cur.xb) >= 0;
-        // flow -> pixels with SCALAR multiplies (see gather_pair)
+        // flow -> pixels with SCALAR multiplies (see gather_pair_packed)
         const float2 fxp = make_float2(__fmul_rn(sx, cur.fx.x), __fmul_rn(sx, cur.fx.y));
         const float2 fyp = make_float2(__fmul_rn(sy, cur.fy.x), __fmul_rn(sy, cur.fy.y));
         GatherPx G2[2];

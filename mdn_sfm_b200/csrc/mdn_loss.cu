@@ -52,7 +52,6 @@ constexpr int S1 = TW + 4, R1H = TH + 2, R1P = S1 * R1H;
 constexpr int WPR = 3;                                      // window rows per SSIM patch (2 columns x WPR rows)
 static_assert((TH + 2) % WPR == 0, "SSIM patches tile the halo-1 region exactly");
 constexpr int NCP = (TW + 2) / 2, NPATCH = NCP * ((TH + 2) / WPR);
-constexpr int RING = W2 * R2H - TW * TH;              // halo slots of the halo-2 region
 constexpr int FUSED_MIN_CTAS = 2;  // 128 registers / thread, no spills; the larger L1 carve-out of 2 CTAs / SM helps the gather
 
 // partial-sum slots per tile
@@ -281,23 +280,6 @@ MDN_DEV void tile_fmat(const KParams& P, int s, int pair, int b, float* F) {
 #pragma unroll
     for (int k = 0; k < 9; ++k) F[k] = __ldg(src + k);
   }
-}
-
-MDN_DEV float post_process(const KParams& P, float e, float snmax, float wgt, float& dpost_de) {
-  // returns post (before the DS mask) and d(post)/d(e); wgt = Gaussian distance weight of the pixel (TG only)
-  if (P.post == MDN_POST_SN) {
-    float q = __fdiv_rn(e, snmax);            // loss_utils.py:98
-    dpost_de = 2.f * q / snmax;
-    return __fmul_rn(q, q);                   // :99
-  }
-  float r = e, dr = 1.f;
-  if (P.threshold > 0.f) {                                                             // loss_utils.py:85-86
-    r = (P.flags & MDN_OPT_CUDA_ARITH) ? __fmul_rn(r, P.inv_threshold) : __fdiv_rn(r, P.threshold);
-    dr = dr * P.inv_threshold;
-  }
-  if (P.post == MDN_POST_TG) { r = __fdiv_rn(r, wgt); dr = dr / wgt; }   // :87-88
-  dpost_de = 2.f * r * dr;
-  return __fmul_rn(r, r);                     // :89
 }
 
 // ----------------------------------------------------------------------------------------------- SN pre-pass

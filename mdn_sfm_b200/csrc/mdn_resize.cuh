@@ -117,14 +117,8 @@ MDN_DEV AaSpan aa_span_no_total(int i, int in_size, float scale) {
   return sp;
 }
 
-MDN_DEV AaSpan aa_span(int i, int in_size, float scale) {
-  AaSpan sp = aa_span_no_total(i, in_size, scale);
-  for (int j = 0; j < sp.xsize; ++j) sp.total = __fadd_rn(sp.total, sp.raw(j));
-  return sp;
-}
-
 // Three launches: the per-axis spans / normalised weights of every output index (a few thousand floats, the only place
-// that needs the double-precision steps of aa_span), then two separable passes as the library does them (the
+// that needs the double-precision steps of aa_span_no_total), then two separable passes as the library does them (the
 // intermediate is rounded to fp32 exactly like ATen's temporary tensor):
 //   H: tmp_k[b][y][ox] = sum_j src[b][y][xmin + j] * wx[j]   for every source row y and every output size k
 //   V: dst_k[b][oy][ox] = round(sum_y tmp_k[b][ymin + y][ox] * wy[y])
