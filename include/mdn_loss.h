@@ -31,7 +31,7 @@ extern "C" {
 #define MDN_API
 #endif
 
-#define MDN_ABI_VERSION 3
+#define MDN_ABI_VERSION 4
 #define MDN_MAX_SCALES 4
 #define MDN_MAX_PAIRS 2
 
@@ -119,10 +119,10 @@ typedef struct MdnLossDesc {
   MdnScale scale[MDN_MAX_SCALES];
   /* Optional pose inputs (since ABI 2).  When cam[p] is given for every pair, the fundamental matrices are built INSIDE the
    * call -- F = K^-T ((t_x R) K^-1), loss_utils.py:50-62, with R = cam[:, :3, :3], t = cam[:, :3, 3]
-   * (loss_functions.py:45-46) and K^-1 = inv_K[s][:, :3, :3] (:123), products accumulated like mdn_fundamental_fwd --
-   * and scale[s].fmat[p] is ignored (may be NULL); inv_K[s] is then required for every scale.  With MDN_OPT_GRADS,
-   * g_cam[p] (may be NULL) receives d(loss)/d(cam[p]): d/dR in [:3,:3], d/dt in [:3,3], zeros elsewhere -- what
-   * mdn_fundamental_bwd would return for the call's d/dF, without the two extra launches. */
+   * (loss_functions.py:45-46) and K^-1 = inv_K[s][:, :3, :3] (:123); each 3x3 product accumulates k = 0,1,2 with FMAs,
+   * the order of the batched SGEMM the reference runs -- and scale[s].fmat[p] is ignored (may be NULL); inv_K[s] is then
+   * required for every scale.  With MDN_OPT_GRADS, g_cam[p] (may be NULL) receives d(loss)/d(cam[p]) through the F of
+   * every scale: d/dR in [:3,:3], d/dt in [:3,3], zeros elsewhere. */
   const float* cam[MDN_MAX_PAIRS];     /* (B,4,4) relative pose target -> source frame p                          */
   float* g_cam[MDN_MAX_PAIRS];         /* (B,4,4)                                                                 */
   const float* inv_K[MDN_MAX_SCALES];  /* (B,4,4) inverse intrinsics of pyramid level s                           */
@@ -193,19 +193,6 @@ MDN_API int mdn_loss_fused_profile(const MdnLossDesc* desc, float* loss_out, voi
  * g == 1) the kernel exits without touching memory.  `g` and `applied` are device scalars.
  */
 MDN_API int mdn_loss_scale_grads(const MdnLossDesc* desc, const float* g, float* applied, void* stream);
-
-/*
- * Fundamental matrices for every (scale, source frame, sample) in one launch: F = K^-T ((t_x R) K^-1),
- * loss_utils.py:50-62, with R = cam[:, :3, :3], t = cam[:, :3, 3] (loss_functions.py:45-46) and
- * K^-1 = inv_K[:, :3, :3] (loss_functions.py:123).  `inv_K` is a HOST array of n_scales device pointers to (B,4,4)
- * matrices, `cam` a HOST array of n_pairs device pointers to (B,4,4) poses; fmat is (n_scales, n_pairs, B, 3, 3).
- * Each 3x3 product accumulates k = 0,1,2 with FMAs, the order of the batched SGEMM the reference runs.
- * The backward takes g_fmat (same shape) and writes g_cam[p] (B,4,4): d/dR in [:3,:3], d/dt in [:3,3], zeros elsewhere.
- */
-MDN_API int mdn_fundamental_fwd(const float* const* inv_K, const float* const* cam, float* fmat, int32_t n_scales,
-                                int32_t n_pairs, int32_t batch, void* stream);
-MDN_API int mdn_fundamental_bwd(const float* const* inv_K, const float* const* cam, const float* g_fmat,
-                                float* const* g_cam, int32_t n_scales, int32_t n_pairs, int32_t batch, void* stream);
 
 /*
  * get_epipolar_new (loss_utils.py:39-69) for arbitrary homogeneous point sets: p1, p2 are (B,3,N), fmat

@@ -20,7 +20,7 @@ WARP_FLOWWARP_NORM, WARP_CUDA_ARITH = 1, 2
 WARP_PAD = {"zeros": 0, "border": 4, "reflection": 8}      # bits 2-3 of warp_flags
 OUT_LOSS, OUT_EPIP, OUT_SMOOTH, OUT_CONSIS, OUT_PHOTO, OUT_APPLIED, OUT_COUNT = 0, 1, 2, 3, 4, 5, 8
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 _P = C.c_void_p
 _PAIR = _P * MAX_PAIRS
@@ -50,7 +50,6 @@ LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_lib", "lib
 
 EXPORTS = ("mdn_version", "mdn_last_error_string", "mdn_loss_workspace_bytes", "mdn_loss_fused", "mdn_loss_fused_profile",
            "mdn_loss_scale_grads",
-           "mdn_fundamental_fwd", "mdn_fundamental_bwd",
            "mdn_epipolar_points_fwd", "mdn_epipolar_points_bwd", "mdn_epipolar_points_workspace_bytes",
            "mdn_flow_warp_fwd", "mdn_flow_warp_bwd", "mdn_ssim_fwd", "mdn_ssim_bwd", "mdn_binary_image",
            "mdn_instance_mask_union", "mdn_instance_mask_union_table", "mdn_instance_mask_resize", "mdn_instance_mask_resize_workspace_bytes", "mdn_image_pyramid", "mdn_image_pyramid_packed", "mdn_normalize_u8",
@@ -75,8 +74,6 @@ class Library:
             "mdn_loss_fused": (C.c_int, [D, _P, _P, sz, _P]),
             "mdn_loss_fused_profile": (C.c_int, [D, _P, _P, sz, _P, C.POINTER(C.c_float)]),
             "mdn_loss_scale_grads": (C.c_int, [D, _P, _P, _P]),
-            "mdn_fundamental_fwd": (C.c_int, [C.POINTER(_P), C.POINTER(_P), _P, i32, i32, i32, _P]),
-            "mdn_fundamental_bwd": (C.c_int, [C.POINTER(_P), C.POINTER(_P), _P, C.POINTER(_P), i32, i32, i32, _P]),
             "mdn_epipolar_points_fwd": (C.c_int, [_P, _P, _P, _P, i32, i64, _P]),
             "mdn_epipolar_points_bwd": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, i32, i64, _P, sz, _P]),
             "mdn_epipolar_points_workspace_bytes": (sz, [i32, i64]),

@@ -101,17 +101,6 @@ struct KParams {
 static_assert(sizeof(KParams) <= 3800, "kernel parameter space");
 
 // ----------------------------------------------------------------------------------------------- fundamental matrix
-struct FundArgs {
-  const float* inv_K[MDN_MAX_SCALES];
-  const float* cam[MDN_MAX_PAIRS];
-  const float* aa[MDN_MAX_PAIRS];      // pose parameters instead of cam (see pose_from_params)
-  const float* tr[MDN_MAX_PAIRS];
-  float* g_cam[MDN_MAX_PAIRS];
-  float* g_aa[MDN_MAX_PAIRS];
-  float* g_tr[MDN_MAX_PAIRS];
-  int n_scales, n_pairs, batch;
-};
-
 // transformation_from_parameters (networks/layers.py:16-98, invert=False as trainer.py:272 calls it): Rodrigues' formula
 // with the reference's operation order and separate roundings -- angle = |v| (:64), axis = v / (angle + 1e-7) (:65), cos /
 // sin (:67-68), C = 1 - cos (:69), the nine entries (:87-95); M = T R (:38) leaves M[:3,:3] = R and M[:3,3] = t exactly
@@ -154,17 +143,15 @@ MDN_DEV void pose_params_bwd(const float* aa, const float* gR, float* g) {
 }
 
 // the (4,4) pose of (pair p, sample b): loaded, or built from the pose parameters
-template <class A>
-MDN_DEV void load_cam(const A& a, int p, int b, float* cam) {
-  if (a.aa[p]) pose_from_params(a.aa[p] + b * 3, a.tr[p] + b * 3, cam);
+MDN_DEV void load_cam(const KParams& P, int p, int b, float* cam) {
+  if (P.aa[p]) pose_from_params(P.aa[p] + b * 3, P.tr[p] + b * 3, cam);
   else {
-    const float* src = a.cam[p] + b * 16;
+    const float* src = P.cam[p] + b * 16;
 #pragma unroll
     for (int k = 0; k < 16; ++k) cam[k] = src[k];
   }
 }
-template <class A>
-MDN_DEV bool has_pose(const A& a, int p) { return a.cam[p] != nullptr || a.aa[p] != nullptr; }
+MDN_DEV bool has_pose(const KParams& P, int p) { return P.cam[p] != nullptr || P.aa[p] != nullptr; }
 
 MDN_DEV void mat3_mul(const float* A, const float* Bm, float* C) {   // C = A B, k-ordered FMA accumulation from 0
 #pragma unroll
@@ -186,8 +173,11 @@ MDN_DEV void load_pose(const float* cam, float* R, float* tx) {   // (4,4) row-m
   tx[0] = 0.f; tx[1] = -t2; tx[2] = t1; tx[3] = t2; tx[4] = 0.f; tx[5] = -t0; tx[6] = -t1; tx[7] = t0; tx[8] = 0.f;
 }
 
-// F = K^-T ((t_x R) K^-1) from M1 = t_x R and the (4,4) inverse intrinsics of one sample (loss_utils.py:61-62)
-MDN_DEV void fundamental_from_m1(const float* M1, const float* kp, float* F) {
+// F = K^-T ((t_x R) K^-1) from the (4,4) pose and the (4,4) inverse intrinsics of one sample (loss_utils.py:61-62)
+MDN_DEV void fundamental_from_pose(const float* cam, const float* kp, float* F) {
+  float R[9], tx[9], M1[9];
+  load_pose(cam, R, tx);
+  mat3_mul(tx, R, M1);                                // loss_utils.py:61
   float K[9], KT[9], M2[9];
 #pragma unroll
   for (int r = 0; r < 3; ++r)
@@ -195,13 +185,6 @@ MDN_DEV void fundamental_from_m1(const float* M1, const float* kp, float* F) {
     for (int c = 0; c < 3; ++c) { K[r * 3 + c] = kp[r * 4 + c]; KT[c * 3 + r] = kp[r * 4 + c]; }
   mat3_mul(M1, K, M2);                                // loss_utils.py:62 (inner product first)
   mat3_mul(KT, M2, F);
-}
-
-MDN_DEV void fundamental_from_pose(const float* cam, const float* kp, float* F) {
-  float R[9], tx[9], M1[9];
-  load_pose(cam, R, tx);
-  mat3_mul(tx, R, M1);                                // loss_utils.py:61
-  fundamental_from_m1(M1, kp, F);
 }
 
 // One scale's term of dL/dM1 = sum_s K gF K^T (K = K^-1 of scale s, kp its (4,4) row-major matrix of the sample)
@@ -213,60 +196,6 @@ MDN_DEV void fundamental_bwd_scale_term(const float* kp, const float* gF, float*
     for (int c = 0; c < 3; ++c) { K[r * 3 + c] = kp[r * 4 + c]; KT[c * 3 + r] = kp[r * 4 + c]; }
   mat3_mul(K, gF, T1);
   mat3_mul(T1, KT, T2);
-}
-
-MDN_DEV void fundamental_bwd_finish(const FundArgs& A, const float* G1, int p, int b);
-
-// d(loss)/d(cam[p][b]) from d(loss)/dF of every scale; g_fmat is [n_scales][n_pairs][batch][9]
-MDN_DEV void fundamental_bwd_one(const FundArgs& A, const float* g_fmat, int p, int b) {
-  float G1[9];
-#pragma unroll
-  for (int k = 0; k < 9; ++k) G1[k] = 0.f;
-  for (int s = 0; s < A.n_scales; ++s) {
-    float T2[9], gF[9];
-    const float* g = g_fmat + ((size_t)(s * A.n_pairs + p) * A.batch + b) * 9;
-#pragma unroll
-    for (int k = 0; k < 9; ++k) gF[k] = __ldcg(g + k);
-    fundamental_bwd_scale_term(A.inv_K[s] + b * 16, gF, T2);
-#pragma unroll
-    for (int k = 0; k < 9; ++k) G1[k] += T2[k];
-  }
-  fundamental_bwd_finish(A, G1, p, b);
-}
-
-// ... from G1 = dL/dM1 (the scale terms added in scale order)
-MDN_DEV void fundamental_bwd_finish(const FundArgs& A, const float* G1, int p, int b) {
-  float R[9], tx[9], cam[16];
-  load_cam(A, p, b, cam);
-  load_pose(cam, R, tx);
-  float txT[9], RT[9], gR[9], gTx[9];
-#pragma unroll
-  for (int r = 0; r < 3; ++r)
-#pragma unroll
-    for (int c = 0; c < 3; ++c) { txT[c * 3 + r] = tx[r * 3 + c]; RT[c * 3 + r] = R[r * 3 + c]; }
-  mat3_mul(txT, G1, gR);                                // M1 = t_x R
-  mat3_mul(G1, RT, gTx);
-  const float gt0 = gTx[7] - gTx[5];                    // t0: t_x[2][1] = t0, t_x[1][2] = -t0
-  const float gt1 = gTx[2] - gTx[6];                    // t1: t_x[0][2] = t1, t_x[2][0] = -t1
-  const float gt2 = gTx[3] - gTx[1];                    // t2: t_x[1][0] = t2, t_x[0][1] = -t2
-  if (A.g_cam[p]) {
-    float* out = A.g_cam[p] + b * 16;
-#pragma unroll
-    for (int k = 0; k < 16; ++k) out[k] = 0.f;
-#pragma unroll
-    for (int r = 0; r < 3; ++r)
-#pragma unroll
-      for (int c = 0; c < 3; ++c) out[r * 4 + c] = gR[r * 3 + c];
-    out[3] = gt0; out[7] = gt1; out[11] = gt2;
-  }
-  // pose parameters given: the adjoint of transformation_from_parameters too (M[:3,3] = t, M[:3,:3] = Rodrigues(axisangle))
-  if (A.aa[p] && A.g_tr[p]) { float* o = A.g_tr[p] + b * 3; o[0] = gt0; o[1] = gt1; o[2] = gt2; }
-  if (A.aa[p] && A.g_aa[p]) {
-    float ga[3];
-    pose_params_bwd(A.aa[p] + b * 3, gR, ga);
-    float* o = A.g_aa[p] + b * 3;
-    o[0] = ga[0]; o[1] = ga[1]; o[2] = ga[2];
-  }
 }
 
 // the fundamental matrix of (scale s, pair, sample b): built from the pose when one was given, else loaded
@@ -407,6 +336,41 @@ struct FParams {
   double inv_N[MDN_MAX_SCALES], inv_div[MDN_MAX_SCALES], inv_cx[MDN_MAX_SCALES], inv_cy[MDN_MAX_SCALES];
 };
 
+// d(loss)/d(pose of pair p, sample b) from G1 = dL/dM1 (the scale terms added in scale order)
+MDN_DEV void fundamental_bwd_finish(const FParams& Q, const float* G1, int p, int b) {
+  float R[9], tx[9], cam[16];
+  load_cam(Q.K, p, b, cam);
+  load_pose(cam, R, tx);
+  float txT[9], RT[9], gR[9], gTx[9];
+#pragma unroll
+  for (int r = 0; r < 3; ++r)
+#pragma unroll
+    for (int c = 0; c < 3; ++c) { txT[c * 3 + r] = tx[r * 3 + c]; RT[c * 3 + r] = R[r * 3 + c]; }
+  mat3_mul(txT, G1, gR);                                // M1 = t_x R
+  mat3_mul(G1, RT, gTx);
+  const float gt0 = gTx[7] - gTx[5];                    // t0: t_x[2][1] = t0, t_x[1][2] = -t0
+  const float gt1 = gTx[2] - gTx[6];                    // t1: t_x[0][2] = t1, t_x[2][0] = -t1
+  const float gt2 = gTx[3] - gTx[1];                    // t2: t_x[1][0] = t2, t_x[0][1] = -t2
+  if (Q.g_cam[p]) {
+    float* out = Q.g_cam[p] + b * 16;
+#pragma unroll
+    for (int k = 0; k < 16; ++k) out[k] = 0.f;
+#pragma unroll
+    for (int r = 0; r < 3; ++r)
+#pragma unroll
+      for (int c = 0; c < 3; ++c) out[r * 4 + c] = gR[r * 3 + c];
+    out[3] = gt0; out[7] = gt1; out[11] = gt2;
+  }
+  // pose parameters given: the adjoint of transformation_from_parameters too (M[:3,3] = t, M[:3,:3] = Rodrigues(axisangle))
+  if (Q.K.aa[p] && Q.g_tr[p]) { float* o = Q.g_tr[p] + b * 3; o[0] = gt0; o[1] = gt1; o[2] = gt2; }
+  if (Q.K.aa[p] && Q.g_aa[p]) {
+    float ga[3];
+    pose_params_bwd(Q.K.aa[p] + b * 3, gR, ga);
+    float* o = Q.g_aa[p] + b * 3;
+    o[0] = ga[0]; o[1] = ga[1]; o[2] = ga[2];
+  }
+}
+
 constexpr int FIN_ROWS = 24;  // FIN_ROWS * NSLOT = 960 threads: at most ~5 tiles per thread at the headline shape
 
 __global__ void __launch_bounds__(FIN_ROWS * NSLOT) finish_kernel(const __grid_constant__ FParams Q) {
@@ -520,16 +484,9 @@ __global__ void __launch_bounds__(FIN_ROWS * NSLOT) finish_kernel(const __grid_c
     }
   }
   __syncthreads();
-  // pose adjoint of this sample (what mdn_fundamental_bwd computes): the scale terms added in scale order, then the
-  // adjoint of M1 = [t]x R and of the pose parameters
+  // pose adjoint of this sample, one thread per pair: d(loss)/dM1 = sum_s K_s gF_s K_s^T (K_s = K^-1 of scale s), the
+  // terms added in scale order, then the adjoint of M1 = [t]x R and of the pose parameters
   if (Q.gf_ws && threadIdx.x < (unsigned)P.n_pairs && (Q.g_cam[threadIdx.x] || Q.g_aa[threadIdx.x] || Q.g_tr[threadIdx.x])) {
-    FundArgs A;
-    for (int k = 0; k < MDN_MAX_SCALES; ++k) A.inv_K[k] = P.inv_K[k];
-    for (int k = 0; k < MDN_MAX_PAIRS; ++k) {
-      A.cam[k] = P.cam[k]; A.aa[k] = P.aa[k]; A.tr[k] = P.tr[k];
-      A.g_cam[k] = Q.g_cam[k]; A.g_aa[k] = Q.g_aa[k]; A.g_tr[k] = Q.g_tr[k];
-    }
-    A.n_scales = P.n_scales; A.n_pairs = P.n_pairs; A.batch = P.batch;
     float G1[9];
 #pragma unroll
     for (int k = 0; k < 9; ++k) G1[k] = 0.f;
@@ -537,7 +494,7 @@ __global__ void __launch_bounds__(FIN_ROWS * NSLOT) finish_kernel(const __grid_c
 #pragma unroll
       for (int k = 0; k < 9; ++k) G1[k] += pose_terms[s][threadIdx.x][k];
     }
-    fundamental_bwd_finish(A, G1, threadIdx.x, b);
+    fundamental_bwd_finish(Q, G1, threadIdx.x, b);
   }
   // last block to arrive folds the per-sample sums into the loss scalars, in a fixed order
   __threadfence();
@@ -690,30 +647,6 @@ __global__ void epipolar_points_bwd_finish_kernel(const float* __restrict__ part
   float t = 0.f;
   for (int j = 0; j < nblk; ++j) t += partials[((long long)b * nblk + j) * EPB_SLOTS + k];
   g_fmat[b * 9 + k] = t;
-}
-
-__global__ void fundamental_fwd_kernel(const __grid_constant__ FundArgs A, float* __restrict__ fmat) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= A.n_pairs * A.batch) return;
-  const int p = i / A.batch, b = i - p * A.batch;
-  float R[9], tx[9], M1[9], cam[16];
-  load_cam(A, p, b, cam);
-  load_pose(cam, R, tx);
-  mat3_mul(tx, R, M1);                                  // loss_utils.py:61
-  for (int s = 0; s < A.n_scales; ++s) {
-    float F[9];
-    fundamental_from_m1(M1, A.inv_K[s] + b * 16, F);
-    float* out = fmat + ((size_t)(s * A.n_pairs + p) * A.batch + b) * 9;
-#pragma unroll
-    for (int k = 0; k < 9; ++k) out[k] = F[k];
-  }
-}
-
-__global__ void fundamental_bwd_kernel(const __grid_constant__ FundArgs A, const float* __restrict__ g_fmat) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= A.n_pairs * A.batch) return;
-  const int p = i / A.batch;
-  fundamental_bwd_one(A, g_fmat, p, i - p * A.batch);
 }
 
 __global__ void __launch_bounds__(NTHREADS) flow_warp_fwd_kernel(const float* __restrict__ ref, const float* __restrict__ flow,
@@ -1205,47 +1138,6 @@ extern "C" MDN_API int mdn_loss_scale_grads(const MdnLossDesc* d, const float* g
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return fail(MDN_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
   return MDN_OK;
-}
-
-static int fund_args(FundArgs& A, const float* const* inv_K, const float* const* cam, float* const* g_cam, int n_scales,
-                     int n_pairs, int batch) {
-  if (!inv_K || !cam) return fail(MDN_ERR_NULL_POINTER, "inv_K / cam pointer array is NULL");
-  if (n_scales < 1 || n_scales > MDN_MAX_SCALES || n_pairs < 1 || n_pairs > MDN_MAX_PAIRS || batch < 1)
-    return fail(MDN_ERR_BAD_SHAPE, "n_scales / n_pairs / batch out of range");
-  memset(&A, 0, sizeof(A));
-  A.n_scales = n_scales; A.n_pairs = n_pairs; A.batch = batch;
-  for (int s = 0; s < n_scales; ++s) { if (!inv_K[s]) return fail(MDN_ERR_NULL_POINTER, "%s is NULL", "inv_K[s]"); A.inv_K[s] = inv_K[s]; }
-  for (int p = 0; p < n_pairs; ++p) {
-    if (!cam[p]) return fail(MDN_ERR_NULL_POINTER, "%s is NULL", "cam[p]");
-    A.cam[p] = cam[p];
-    if (g_cam) { if (!g_cam[p]) return fail(MDN_ERR_NULL_POINTER, "%s is NULL", "g_cam[p]"); A.g_cam[p] = g_cam[p]; }
-  }
-  return MDN_OK;
-}
-
-extern "C" MDN_API int mdn_fundamental_fwd(const float* const* inv_K, const float* const* cam, float* fmat, int32_t n_scales,
-                                           int32_t n_pairs, int32_t batch, void* stream) {
-  FundArgs A;
-  int rc = fund_args(A, inv_K, cam, nullptr, n_scales, n_pairs, batch);
-  if (rc != MDN_OK) return rc;
-  if (!fmat) return fail(MDN_ERR_NULL_POINTER, "fmat is NULL");
-  const int n = n_pairs * batch;
-  MDN_LAUNCH(fundamental_fwd_kernel, dim3((n + 63) / 64), dim3(64), 0, (cudaStream_t)stream, A, fmat);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? MDN_OK : fail(MDN_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
-}
-
-extern "C" MDN_API int mdn_fundamental_bwd(const float* const* inv_K, const float* const* cam, const float* g_fmat,
-                                           float* const* g_cam, int32_t n_scales, int32_t n_pairs, int32_t batch, void* stream) {
-  FundArgs A;
-  if (!g_cam) return fail(MDN_ERR_NULL_POINTER, "g_cam pointer array is NULL");
-  int rc = fund_args(A, inv_K, cam, g_cam, n_scales, n_pairs, batch);
-  if (rc != MDN_OK) return rc;
-  if (!g_fmat) return fail(MDN_ERR_NULL_POINTER, "g_fmat is NULL");
-  const int n = n_pairs * batch;
-  MDN_LAUNCH(fundamental_bwd_kernel, dim3((n + 63) / 64), dim3(64), 0, (cudaStream_t)stream, A, g_fmat);
-  cudaError_t e = cudaGetLastError();
-  return e == cudaSuccess ? MDN_OK : fail(MDN_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(e));
 }
 
 static inline unsigned blocks_for(long long n, int cap = 148 * 8) {

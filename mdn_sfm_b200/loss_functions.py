@@ -33,7 +33,6 @@ from .layers import SSIM, PoseParameters, get_scale_factor  # noqa: F401  (re-ex
 from .loss_utils import *  # noqa: F401,F403  (the reference does `from loss_utils import *`)
 from .loss_utils import create_coords as _create_coords
 from .loss_utils import _arith_flag, instance_mask_u8, instance_masks_u8
-from .ops import fundamental_matrices
 from .utils import gauss_distance_weight
 
 MODES = ("SN", "T", "TG", "DS", "DC")
@@ -250,9 +249,6 @@ class Loss(nn.Module):
         self._library = library
         self._arith = arith
         self._cuda_arith = _arith_flag(arith)
-        # arith="cuda": hand the poses to the fused call (F and the pose gradients are computed inside it) instead of
-        # running the fundamental-matrix prologue / epilogue kernels around it; False keeps the three-launch form
-        self.pose_in = True
         self._helper = None
 
     def _lm(self):
@@ -266,7 +262,7 @@ class Loss(nn.Module):
         ids = list(frame_id)
         poses = None
         params = all(isinstance(cam_T_cam[i], PoseParameters) for i in ids)
-        if params and not (self._cuda_arith and self.pose_in):
+        if params and not self._cuda_arith:
             cam_T_cam = {i: cam_T_cam[i].matrix() for i in ids}      # the torch composition of networks/layers.py:16-98
             params = False
         if params:
@@ -276,13 +272,9 @@ class Loss(nn.Module):
             trs = [_c(cam_T_cam[i].translation, "translation") for i in ids]
             inv_Ks = [_c(inputs[("inv_K", s)].detach(), "inv_K") for s in scales]
             poses = ("params", aas, trs, inv_Ks)
-        elif self._cuda_arith and not self.pose_in:
-            # one prologue launch (mdn_fundamental_fwd): F for every (scale, source frame, sample); autograd carries
-            # d/dF back to the poses through mdn_fundamental_bwd.  Same arithmetic as the in-kernel path below.
-            F_all = fundamental_matrices([inputs[("inv_K", s)] for s in scales], [cam_T_cam[i] for i in ids], self._library)
         elif self._cuda_arith:
             # the kernels build F themselves from the poses (MdnLossDesc.cam / inv_K: 3x3 products accumulated like the
-            # batched SGEMM the reference runs on CUDA) and return the pose gradients: no prologue / epilogue launches
+            # batched SGEMM the reference runs on CUDA) and return the pose gradients
             F_all = None
             cams = [_c(cam_T_cam[i], "cam_T_cam") for i in ids]
             inv_Ks = [_c(inputs[("inv_K", s)].detach(), "inv_K") for s in scales]

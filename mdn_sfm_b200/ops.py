@@ -98,39 +98,3 @@ class SsimFn(torch.autograd.Function):
                          _cabi.ptr(gy), planes, h, w, _cabi.stream_ptr(x), dev=x)
         return gx, gy, None
 
-
-class FundamentalFn(torch.autograd.Function):
-    """F[s, p] = K_s^-T ((t_x R)_p K_s^-1) for every scale and source frame in one launch (loss_utils.py:50-62).
-
-    apply(n_scales, library, inv_K_0 .. inv_K_{S-1}, cam_0 .. cam_{P-1}) -> (S, P, B, 3, 3); gradients flow to the poses.
-    """
-
-    @staticmethod
-    def forward(ctx, n_scales, library, *mats):
-        library = library or _cabi.lib()
-        inv_K, cams = list(mats[:n_scales]), list(mats[n_scales:])
-        B = cams[0].shape[0]
-        fmat = torch.empty((n_scales, len(cams), B, 3, 3), dtype=torch.float32, device=cams[0].device)
-        library.call("mdn_fundamental_fwd", _cabi.ptr_array(inv_K), _cabi.ptr_array(cams), fmat.data_ptr(), n_scales,
-                     len(cams), B, _cabi.stream_ptr(fmat), dev=fmat)
-        ctx.library, ctx.n_scales, ctx.mats = library, n_scales, (inv_K, cams)
-        return fmat
-
-    @staticmethod
-    def backward(ctx, g):
-        inv_K, cams = ctx.mats
-        g = g.contiguous()
-        g_cam = [torch.empty_like(c) for c in cams]
-        ctx.library.call("mdn_fundamental_bwd", _cabi.ptr_array(inv_K), _cabi.ptr_array(cams), g.data_ptr(),
-                         _cabi.ptr_array(g_cam), ctx.n_scales, len(cams), cams[0].shape[0], _cabi.stream_ptr(g), dev=g)
-        return (None, None) + (None,) * ctx.n_scales + tuple(g_cam)
-
-
-def fundamental_matrices(inv_K_list, cam_list, library=None):
-    """inv_K_list: S tensors (B,4,4); cam_list: P tensors (B,4,4) -> (S,P,B,3,3)."""
-    inv_K = [_c(k.detach(), "inv_K") for k in inv_K_list]
-    cams = [_c(c, "cam_T_cam") for c in cam_list]
-    for t in inv_K + cams:
-        if t.dim() != 3 or tuple(t.shape[1:]) != (4, 4):
-            raise ValueError("inv_K / cam_T_cam must be (B,4,4)")
-    return FundamentalFn.apply(len(inv_K), library, *inv_K, *cams)

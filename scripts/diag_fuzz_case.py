@@ -18,7 +18,7 @@ batch = synthetic.make_batch(B, H, W, scales=scales, seed=c["seed"], flow_std=c[
 if c["kind"] != "inst":
     batch = batch[:4] + (None,)
 ref = common.oracle_run(opt, batch, mode, c["photo"], c["ssim"], device="cuda", pose_grad=True, padding_mode=c["pad"])
-got = common.product_run(opt, batch, mode, c["photo"], c["ssim"], "cuda", pose_grad=True, pose_in=c["pose_in"], padding_mode=c["pad"])
+got = common.product_run(opt, batch, mode, c["photo"], c["ssim"], "cuda", pose_grad=True, padding_mode=c["pad"])
 # float64 oracle for the pose gradients (the reference's own fp32 noise floor)
 torch.set_default_dtype(torch.float64)
 b64 = tuple(({k: v.double() for k, v in d.items()} if isinstance(d, dict) else d) for d in batch)

@@ -39,17 +39,16 @@ def main():
         dmin, dsm, dcs = rng.random() < 0.3, rng.random() < 0.2, rng.random() < 0.2
         fstd = rng.choice([0.01, 0.05, 0.2, 0.6])
         pad = rng.choice(["zeros", "zeros", "zeros", "border", "reflection"])
-        pose_in = rng.random() < 0.7
         seed = rng.randint(0, 10 ** 6)
         case = dict(kind=kind, B=B, H=H, W=W, scales=scales, mode=mode, photo=photo, ssim=ssim, dmin=dmin, dsm=dsm, dcs=dcs, fstd=fstd,
-                    pad=pad, pose_in=pose_in, seed=seed)
+                    pad=pad, seed=seed)
         try:
             opt = synthetic.default_opt(B, H, W, disable_min=dmin, disable_smoothloss=dsm, disable_consisloss=dcs, scales=list(scales))
             batch = synthetic.make_batch(B, H, W, scales=scales, seed=seed, flow_std=fstd, with_instances=kind == "inst")
             if kind != "inst":
                 batch = batch[:4] + (None,)
             ref = common.oracle_run(opt, batch, mode, photo, ssim, device="cuda", pose_grad=True, padding_mode=pad)
-            got = common.product_run(opt, batch, mode, photo, ssim, "cuda", pose_grad=True, pose_in=pose_in, padding_mode=pad)
+            got = common.product_run(opt, batch, mode, photo, ssim, "cuda", pose_grad=True, padding_mode=pad)
             # B = 1: the reference's own CUDA result depends on the batch size there (torch.matmul runs gemm for one batch, bgemm for
             # more; scripts/diag_batch1.py: its distance maps differ by 2e-5 ... 5e-5 between B = 1 and the same sample in a batch
             # of two).  The product follows the B >= 2 rounding at every batch size, so B = 1 is compared at that noise floor.

@@ -1,6 +1,6 @@
 """Kernel-variant timing: python scripts/kbench.py lib1.so [lib2.so ...] [--shape HxW] [--batch B] [--mode T] [--iters N]
 
-Times Loss.forward (= fundamental prologue + mdn_loss_fused) with CUDA events over 4 rotating input sets for each
+Times Loss.forward (= mdn_loss_fused, F built in the call from the poses) with CUDA events over 4 rotating input sets for each
 library build given on the command line (any builds of libmdn_loss.so, for example of two commits).  Experiment
 tooling: bench.py is the number of record.
 """

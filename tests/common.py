@@ -115,8 +115,7 @@ def _oracle_run(opt, batch, mode, photo, ssim_on, device="cpu", pose_grad=False,
     return out, losses, f, m, cams
 
 
-def product_run(opt, batch, mode, photo, ssim_on, device, pose_grad=False, library=None, arith=None, pose_in=True,
-                padding_mode="zeros"):
+def product_run(opt, batch, mode, photo, ssim_on, device, pose_grad=False, library=None, arith=None, padding_mode="zeros"):
     arith = arith or ("cuda" if str(device).startswith("cuda") else "cpu")
     from mdn_sfm_b200.loss_functions import Loss
     inputs, flows, mobiles, cams, inst = batch
@@ -129,7 +128,6 @@ def product_run(opt, batch, mode, photo, ssim_on, device, pose_grad=False, libra
         cams = leaf(cams)
     scales = sorted({k[2] for k in flows})
     loss = Loss(opt, no_ssim=not ssim_on, padding_mode=padding_mode, mode=mode, photometric=photo, library=library, arith=arith)
-    loss.pose_in = pose_in
     out, losses = loss(inputs, [-1, 1], f, m, inst, scales, cams)
     losses["loss"].backward()
     return out, losses, f, m, cams

@@ -194,33 +194,6 @@ def test_free_functions():
     assert torch.equal(loss_utils.create_coords(2, 5, 7), restate.create_coords(2, 5, 7))
 
 
-def test_fundamental_matrix_prologue():
-    """mdn_fundamental_fwd/bwd vs the reference's three matmuls (loss_utils.py:50-62) and their autograd."""
-    from mdn_sfm_b200 import fused
-    from mdn_sfm_b200.ops import fundamental_matrices
-    g = torch.Generator().manual_seed(2)
-    B, S, P = 3, 4, 2
-    cams = [synthetic.make_pose(torch.randn(B, 1, 1, 3, generator=g) * 0.05, torch.randn(B, 1, 1, 3, generator=g) * 0.2)
-            for _ in range(P)]
-    Ks = []
-    for s in range(S):
-        K = torch.tensor([[0.58 * 640 / 2 ** s, 0, 320 / 2 ** s, 0], [0, 1.92 * 192 / 2 ** s, 96 / 2 ** s, 0],
-                          [0, 0, 1, 0], [0, 0, 0, 1]], dtype=torch.float32)
-        Ks.append(torch.linalg.pinv(K).unsqueeze(0).repeat(B, 1, 1))
-    wgt = torch.randn(S, P, B, 3, 3, generator=g)
-    co = [c.clone().requires_grad_(True) for c in cams]
-    Fo = torch.stack([torch.stack([restate.fundamental_matrix(Ks[s][:, :3, :3], co[p][:, :3, :3], co[p][:, :3, -1])
-                                   for p in range(P)]) for s in range(S)])
-    (Fo * wgt).sum().backward()
-    with emulated():
-        cg = [c.clone().requires_grad_(True) for c in cams]
-        Fg = fundamental_matrices(Ks, cg)
-        (Fg * wgt).sum().backward()
-    assert Fg.shape == Fo.shape and common.rel_max(Fo, Fg) < 1e-5
-    for a, b in zip(co, cg):
-        assert common.rel_max(a.grad, b.grad) < 1e-4
-
-
 def test_multiple_tiles_in_x_and_vector_staging():
     # 136 = two full 64-wide tiles + a ragged one (w % 4 == 0: 16-byte staging path); 68 at scale 1; heights 24 / 12
     opt, batch = common.make(1, 24, 136, scales=(0, 1), seed=17, flow_std=0.06)
@@ -232,17 +205,17 @@ def test_multiple_tiles_in_x_and_vector_staging():
 
 
 @pytest.mark.parametrize("mode", ["SN", "T"])
-def test_poses_inside_the_call_equal_the_prologue_kernels(mode):
-    """MdnLossDesc.cam / inv_K (F and the pose adjoint computed inside mdn_loss_fused) is bit-identical to
-    mdn_fundamental_fwd -> mdn_loss_fused(fmat) -> mdn_fundamental_bwd, two scales, ragged tiles, SN fix-up included."""
+def test_poses_inside_the_call_match_the_oracle(mode):
+    """MdnLossDesc.cam / inv_K: F and the pose adjoint computed inside mdn_loss_fused, two scales, ragged tiles, SN fix-up
+    included.  d/dcam (the g_cam write of the finish kernel) and the loss scalars against the CPU oracle."""
     opt, batch = common.make(2, 24, 72, scales=(0, 1), seed=13, flow_std=0.08)
     with emulated():
-        a = common.product_run(opt, batch, mode, True, True, "cpu", pose_grad=True, arith="cuda", pose_in=True)
-        b = common.product_run(opt, batch, mode, True, True, "cpu", pose_grad=True, arith="cuda", pose_in=False)
-        assert all(c.grad is not None and float(c.grad.abs().sum()) > 0 for c in a[4].values())
-        common.assert_identical_runs(a, b)   # (the per-pixel maps are evaluated lazily: inside the emulated block)
-    # and the CUDA-eager arithmetic stays within tolerance of the CPU oracle away from flipped bilinear cells (scalars only)
+        a = common.product_run(opt, batch, mode, True, True, "cpu", pose_grad=True, arith="cuda")
+    assert all(c.grad is not None and float(c.grad.abs().sum()) > 0 for c in a[4].values())
     ref = common.oracle_run(opt, batch, mode, True, True, pose_grad=True)
+    for k in ref[4]:
+        assert common.rel_max(ref[4][k].grad, a[4][k].grad) <= common.GRAD_TOL, ("d/dcam", k, common.rel_max(ref[4][k].grad, a[4][k].grad))
+    # the CUDA-eager arithmetic stays within tolerance of the CPU oracle away from flipped bilinear cells (scalars only)
     for k in ("loss", "epip", "smooth", "consis", "photo"):
         assert float(a[1][k]) == pytest.approx(float(ref[1][k]), rel=1e-4), k
 

@@ -238,8 +238,8 @@ def test_single_source_frame_with_disable_min():
 
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs in one process")
 def test_every_entry_point_on_a_non_current_device():
-    """cuda:0 is current, the tensors live on cuda:1: DC / DS (instance-mask kernels), the prologue form (pose_in=False),
-    the pyramid producer, uint8 frames, the standalone ops -- every launch must go to the tensors' device."""
+    """cuda:0 is current, the tensors live on cuda:1: DC / DS (instance-mask kernels), the pyramid producer, uint8
+    frames, the standalone ops -- every launch must go to the tensors' device."""
     from mdn_sfm_b200 import loss_utils, pyramid, utils
     torch.cuda.set_device(0)
     opt, batch = common.make(2, 64, 128, seed=5)
@@ -249,9 +249,6 @@ def test_every_entry_point_on_a_non_current_device():
         assert torch.equal(a[1]["loss"].cpu(), b[1]["loss"].cpu()), mode
         for k in a[2]:
             assert torch.equal(a[2][k].grad.cpu(), b[2][k].grad.cpu()), (mode, k)
-    a = common.product_run(opt, batch, "T", True, True, "cuda:0", pose_grad=True, pose_in=False)
-    b = common.product_run(opt, batch, "T", True, True, "cuda:1", pose_grad=True, pose_in=False)
-    assert torch.equal(a[1]["loss"].cpu(), b[1]["loss"].cpu())
     img = batch[0][("color", 0, 0)]
     p0 = pyramid.image_pyramid(img.to("cuda:0"), [(32, 64), (16, 32)])
     p1 = pyramid.image_pyramid(img.to("cuda:1"), [(32, 64), (16, 32)])
